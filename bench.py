@@ -370,11 +370,13 @@ def run_gpu_arm(args, rank, local_rank, world):
         barrier()
         ev0.record()
         for i in range(args.steps):
-            step_device(i)
+            last = step_device(i)
         ev1.record()
         barrier()
     ms = ev0.elapsed_time(ev1)
     launches = lib.azg_launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     phase = {}
     for pid, name in ((0, "trunk"), (1, "gemm"), (2, "heads")):
         tot, cnt = C.c_double(), C.c_int()
@@ -593,6 +595,25 @@ def run_gpu_arm(args, rank, local_rank, world):
         shutdown_ranks(net)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(folder, out):
+    """Writes the device outputs of one step ({name: [B, ...] tensor}) as `folder`/<name>.npy in float32, so that two builds
+    can be compared output for output.  Above 64 MB in all, the same seeded sample of rows is kept from every output."""
+    import numpy as np
+    arrays = {k: v.float().cpu().numpy() for k, v in out.items()}
+    rows = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a.nbytes // max(a.shape[0], 1) for a in arrays.values())
+    budget = DUMP_LIMIT_BYTES - 4096 * len(arrays)  # room for the .npy headers
+    if rows * row_bytes > budget:
+        keep = np.sort(np.random.default_rng(0).choice(rows, budget // row_bytes, replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(folder, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(folder, k + ".npy"), np.ascontiguousarray(a))
+
+
 def shutdown_ranks(*wrappers):
     """Leave a multi-rank run without hanging: graphs that captured NCCL kernels are destroyed first (NCCL's rule), all
     ranks meet at a barrier, and the interpreter is left through os._exit so that no late destructor can block a rank that
@@ -626,7 +647,11 @@ def main():
     ap.add_argument("--cpu-selfplay-episodes", type=int, default=2)
     ap.add_argument("--train-epochs", type=int, default=60, help="timed epochs (std step + GNN step) of NeuralNet.train; 0 = skip")
     ap.add_argument("--coach-eps", type=int, default=4096, help="self-play episodes per GPU of the Coach-iteration leg; 0 = skip")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write pi, v, pi_gnn, v_gnn of the last timed step (rank 0) as DIR/<name>.npy, float32, at most 64 MB")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -15,7 +15,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 REF = os.environ.get("AZG_REFERENCE", "/root/reference")
-sys.path[:0] = [REF, os.path.join(HERE, "_shims"), ROOT]
+sys.path[:0] = [REF, os.path.join(HERE, "_shims"), ROOT, os.path.dirname(HERE)]
 
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
@@ -465,6 +465,16 @@ def gen_reference_files():
         for p_ in list(w.nnet.parameters()) + list(w.gnn.parameters()):
             p_.add_(0.01 * torch.randn_like(p_))
     w.save_checkpoint(folder, "best_gnn.pth.tar")
+    # kept as the file with its tensor records zeroed + the file's SHA-256; tests/helpers.py reference_checkpoint() draws the
+    # weights again from the seed above and restores the file byte for byte
+    import hashlib
+    from helpers import zero_tensor_records
+    ckpt = os.path.join(folder, "best_gnn.pth.tar")
+    with open(ckpt, "rb") as f:
+        buf = f.read()
+    np.savez_compressed(ckpt + ".npz", zeroed=np.frombuffer(bytes(zero_tensor_records(buf)), dtype=np.uint8),
+                        sha256=np.array(hashlib.sha256(buf).hexdigest()))
+    os.remove(ckpt)
     rng = np.random.default_rng(3)
     boards = random_boards(3, 16, rng)
     pis, vs, gpis, gvs = [], [], [], []

@@ -1,5 +1,9 @@
 """Shared test helpers: seeded weight construction, golden loading, MCTS dict dumps."""
+import hashlib
+import io
 import os
+import struct
+import zipfile
 
 import numpy as np
 import torch
@@ -42,6 +46,52 @@ def seeded_two_player_modules(kind, n, seed=0, gnn_layers=2):
 def seeded_fl_module(n, layers, seed=0):
     torch.manual_seed(seed)
     return modules.FrozenLakeGraphNet((n, n), 4, embedding_dim=128, gnn_layers=layers)
+
+
+def tensor_records(buf):
+    """(offset, size) of every tensor record `<archive>/data/<k>` of a torch.save zip file, in the order of k."""
+    recs = []
+    for info in zipfile.ZipFile(io.BytesIO(bytes(buf))).infolist():
+        key = info.filename.rpartition("/data/")[2]
+        if key.isdigit():
+            assert info.compress_type == zipfile.ZIP_STORED, info.filename
+            name_len, extra_len = struct.unpack_from("<HH", buf, info.header_offset + 26)  # zip local file header
+            recs.append((int(key), info.header_offset + 30 + name_len + extra_len, info.file_size))
+    return [(off, size) for _, off, size in sorted(recs)]
+
+
+def zero_tensor_records(buf):
+    """The file with its tensor bytes set to zero (what ref_files/best_gnn.pth.tar.npz stores)."""
+    out = bytearray(buf)
+    for off, size in tensor_records(out):
+        out[off:off + size] = bytes(size)
+    return out
+
+
+def reference_checkpoint(folder):
+    """Writes the reference wrapper's TicTacToe 3x3 checkpoint (`{'state_dict','gnn'}`, 2 MB, make_golden.py
+    gen_reference_files) to `folder`/best_gnn.pth.tar and returns the file name.  The repository keeps that file with its
+    tensor records zeroed; the weights are the seed-5 initialisation plus 0.01 * randn, so they are drawn again here and
+    written back into their records, and the result must hash to the file the reference wrote."""
+    g = np.load(os.path.join(GOLDEN, "ref_files", "best_gnn.pth.tar.npz"), allow_pickle=False)
+    buf = bytearray(g["zeroed"].tobytes())
+    with torch.random.fork_rng(devices=[]), torch.no_grad():  # leaves the caller's RNG state as it was
+        nnet, gnn = seeded_two_player_modules("ttt", 3, seed=5)
+        for p in list(nnet.parameters()) + list(gnn.parameters()):
+            p.add_(0.01 * torch.randn_like(p))
+    tensors = list(nnet.state_dict().values()) + list(gnn.state_dict().values())
+    recs = tensor_records(buf)
+    assert len(recs) == len(tensors)
+    for (off, size), t in zip(recs, tensors):
+        data = t.contiguous().numpy().tobytes()
+        assert len(data) == size
+        buf[off:off + size] = data
+    assert hashlib.sha256(buf).hexdigest() == str(g["sha256"]), "rebuilt checkpoint differs from the reference's file"
+    name = "best_gnn.pth.tar"
+    os.makedirs(folder, exist_ok=True)
+    with open(os.path.join(folder, name), "wb") as f:
+        f.write(buf)
+    return name
 
 
 def checksum_rows(sd):

@@ -23,7 +23,7 @@ from azgnn_b200.coach import Coach  # noqa: E402
 from azgnn_b200.replay import symmetry_tables  # noqa: E402
 from oracle import nets as onets  # noqa: E402
 from oracle.mcts import FakeNet  # noqa: E402
-from helpers import GOLDEN, dotdict, golden  # noqa: E402
+from helpers import GOLDEN, dotdict, golden, reference_checkpoint  # noqa: E402
 
 QT_F32, QT_FLOAT, QT_INT = 0, 1, 2
 
@@ -168,12 +168,14 @@ def test_learn_skips_first_self_play_after_loading(tmp_path, monkeypatch):
     assert played == [1] and Net.trained_on[0] > 0
 
 
-def test_reference_checkpoint_matches_the_parameter_schema():
+def test_reference_checkpoint_matches_the_parameter_schema(tmp_path):
     """The reference's `{'state_dict', 'gnn'}` file (TicTacToeGNN.py save_checkpoint) loads into modules.* with strict key
     and shape matching, and the oracle forward on those weights reproduces the predictions the reference wrapper made
     before saving."""
     idx = golden("ref_files_index")
-    ck = torch.load(os.path.join(GOLDEN, "ref_files", str(idx["checkpoint_file"])), map_location="cpu")
+    name = reference_checkpoint(str(tmp_path))
+    assert name == str(idx["checkpoint_file"])
+    ck = torch.load(os.path.join(str(tmp_path), name), map_location="cpu")
     assert set(ck.keys()) == {"state_dict", "gnn"}
     nnet, gnn = modules.TicTacToeTrunk(3, 10), modules.PolicyValueGNN(128, 2)
     assert sorted(nnet.state_dict().keys()) == [str(x) for x in idx["nnet_names"]]

@@ -13,7 +13,7 @@ import torch
 from azgnn_b200 import games
 from azgnn_b200.coach import Coach
 from azgnn_b200.nets import B200TicTacToeGNNWrapper
-from helpers import GOLDEN, dotdict, golden
+from helpers import GOLDEN, dotdict, golden, reference_checkpoint
 from test_examples_golden import _check_episode
 
 pytestmark = pytest.mark.gpu
@@ -29,10 +29,12 @@ def _wrapper(precision):
 @pytest.mark.parametrize("precision", ["fp32", "auto"])
 def test_reference_checkpoint_loads_and_predicts(precision, tmp_path):
     idx = golden("ref_files_index")
+    ref_dir = str(tmp_path / "reference")
+    assert reference_checkpoint(ref_dir) == str(idx["checkpoint_file"])
     w = _wrapper(precision)
     before = w.predict_batch(idx["boards"])
     assert np.abs(before["pi"] - idx["pi"]).max() > 1e-3
-    w.load_checkpoint(REF_FILES, str(idx["checkpoint_file"]))
+    w.load_checkpoint(ref_dir, str(idx["checkpoint_file"]))
     out = w.predict_batch(idx["boards"])
     for key, want in (("pi", idx["pi"]), ("v", idx["v"]), ("pi_gnn", idx["gnn_pi"]), ("v_gnn", idx["gnn_v"])):
         np.testing.assert_allclose(out[key].reshape(want.shape), want, rtol=0, atol=1e-5, err_msg=key)
@@ -42,7 +44,7 @@ def test_reference_checkpoint_loads_and_predicts(precision, tmp_path):
     # and back: the wrapper's own file has the reference file's structure
     w.save_checkpoint(str(tmp_path), "best_gnn.pth.tar")
     mine = torch.load(str(tmp_path / "best_gnn.pth.tar"), map_location="cpu")
-    ref = torch.load(os.path.join(REF_FILES, str(idx["checkpoint_file"])), map_location="cpu")
+    ref = torch.load(os.path.join(ref_dir, str(idx["checkpoint_file"])), map_location="cpu")
     assert list(mine.keys()) == list(ref.keys()) == ["state_dict", "gnn"]
     for part in ("state_dict", "gnn"):
         assert list(mine[part].keys()) == list(ref[part].keys())
