@@ -13,12 +13,12 @@
 //   * Persistent, warp-specialised kernel: warp 0 = bulk-copy producer, warp 1 = MMA issuer (a single thread
 //     issues tcgen05.mma), warp 2 = TMEM allocator, warps 4-7 = epilogue (tcgen05.ld -> bias/ReLU -> store).
 //     Accumulators live in TMEM, double-buffered (2 x BN fp32 columns) so the epilogue of tile i overlaps the
-//     main loop of tile i+1.  Two instantiations per tile width:
-//       TWO = 0  one CTA per SM, M=128 x N=BN x K=16 MMAs, smem ring of 4 stages x (16 KB A + BN*128 B W);
-//       TWO = 1  CTA pairs (cluster of 2, cta_group::2): 256 x BN x 16 MMAs issued by the leader CTA, each CTA holds
-//                128 rows of A and of the accumulator and BN/2 rows of the weight tile; a stage carries two operand
-//                pairs (bf16x3: hi and lo of one k-block -> all three products; bf16: two k-blocks).  This is the
-//                kernel of the Connect4 F x F contractions; it can also carry a 32-column side tile per m-unit
+//     main loop of tile i+1.  One instantiation per tile width:
+//       TWO = 0  (BN = 64) one CTA per SM, M=128 x N=BN x K=16 MMAs, smem ring of 4 stages x (16 KB A + BN*128 B W);
+//       TWO = 1  (BN >= 128) CTA pairs (cluster of 2, cta_group::2): 256 x BN x 16 MMAs issued by the leader CTA, each
+//                CTA holds 128 rows of A and of the accumulator and BN/2 rows of the weight tile; a stage carries two
+//                operand pairs (bf16x3: hi and lo of one k-block -> all three products; bf16: two k-blocks).  This is
+//                the kernel of the Connect4 F x F contractions; it can also carry a 32-column side tile per m-unit
 //                (GemmArgs::side_*: the standard policy/value heads ride on GEMM-1).
 //   * AZG_PREC_BF16X3 (the 1e-5 parity mode): x = hi + lo with hi = bf16(x), lo = bf16(x - hi);
 //     X W^T ~= Xhi Whi^T + Xhi Wlo^T + Xlo Whi^T, fp32 accumulate.  Implemented as ONE GEMM with a
@@ -34,7 +34,7 @@
 namespace tc {
 
 // ---- epilogue output modes -----------------------------------------------------------------
-enum { OUT_F32 = 0, OUT_IMG = 1, OUT_IMG_HILO = 2, OUT_FEAT = 3, OUT_FEAT_HILO = 4, OUT_HEADS = 5 };
+enum { OUT_F32 = 0, OUT_IMG = 1, OUT_IMG_HILO = 2, OUT_HEADS = 3 };
 constexpr int HEAD_ROWS = 10;    // <= 9 policy logits + 1 value (Connect4 n <= 8)
 constexpr int HEAD_STRIDE = 16;  // floats per (row, n-tile) record of partial head sums
 
@@ -63,9 +63,6 @@ struct GemmArgs {
   float* head_part;     // OUT_HEADS: [M, n_tiles, HEAD_STRIDE] partial sums, reduced in fixed order by heads_finalize
   int head_rows;
   const int32_t* dyn_rows;  // optional device scalar: number of valid rows this launch (<= M), read by the kernel
-  int pair_ok;          // the A image covers an even number of m-tiles: the CTA-pair kernel may be used
-  int feat_nn;          // OUT_FEAT*: rows are (board b, cell p) pairs, m = b*feat_nn + p; the 64 columns (conv2
-                        // channels) become k-block p of row b of the feature image  [K' = p*64 + co]
   // optional side tile (CTA-pair kernel only): one more n-tile of SIDE_N columns per m-unit contracts the same A rows
   // with a second, narrow weight image and writes fp32 [M, SIDE_N] (no ReLU) -- the standard policy/value heads of
   // `predict` ride on GEMM-1 instead of re-reading the feature image in their own launch
@@ -258,24 +255,6 @@ __device__ __forceinline__ void epilogue_tile(const GemmArgs& g, uint32_t taddr,
               hacc[a] = s;
             }
           }
-        } else if (g.out_mode >= OUT_FEAT) {
-          if (row < g.M) {
-            const int64_t bidx = row / g.feat_nn;
-            const int p = (int)(row - bidx * g.feat_nn);
-            const size_t tile = ((size_t)(bidx >> 7) * g.feat_nn + p) * A_STAGE_BYTES;
-            const int rb = (int)(bidx & 127);
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-              uint32_t hi[4], lo[4];
-#pragma unroll
-              for (int e = 0; e < 4; ++e) {
-                split_pair(v[c * 8 + 2 * e], v[c * 8 + 2 * e + 1], hi[e], lo[e]);
-              }
-              const size_t off = tile + image_offset(rb, c0 + c * 8);
-              *reinterpret_cast<uint4*>(g.out_hi + off) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-              if (g.out_mode == OUT_FEAT_HILO) *reinterpret_cast<uint4*>(g.out_lo + off) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-            }
-          }
         } else if (g.out_mode == OUT_F32) {
           if (row < g.M) {
             float4* dst = reinterpret_cast<float4*>(g.out_f32 + row * (int64_t)(g.n_tiles * BN) + n0);
@@ -345,7 +324,7 @@ __global__ void __launch_bounds__(GEMM_THREADS, 1) gemm_bf16_tc_kernel(GemmArgs 
   constexpr uint32_t TMEM_COLS = 512;  // 2 accumulator stages of BN <= 256 fp32 columns
   const uint32_t rank = TWO ? cluster_ctarank() : 0u;
   if (g.dyn_rows) {  // row count decided on the device (compacted leaf batches): no host round trip
-    const int64_t rows = (int64_t)(*g.dyn_rows) * (g.out_mode >= OUT_FEAT && g.out_mode != OUT_HEADS ? g.feat_nn : 1);
+    const int64_t rows = *g.dyn_rows;
     if (rows < g.M) g.M = rows;
     g.m_tiles = (int)((g.M + BM - 1) / BM);
   }
@@ -702,15 +681,6 @@ static int f8_terms() {  // AZG_F8_TERMS=1 / 2: only the fp16 product / only the
   return terms;
 }
 
-static int gemm_pair_mode() {  // AZG_GEMM=1cta disables the CTA-pair kernels (A/B measurements)
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("AZG_GEMM");
-    mode = (e && strcmp(e, "1cta") == 0) ? 0 : 1;
-  }
-  return mode;
-}
-
 template <int BN, bool TWO>
 int launch_gemm_impl(const GemmArgs& g, cudaStream_t st) {
   static bool configured = false;
@@ -748,25 +718,24 @@ int launch_gemm_impl(const GemmArgs& g, cudaStream_t st) {
 // double-buffered and the epilogue (tens of thousands of cycles per tile, see the epilogue comment in gemm_bf16_tc_kernel)
 // is exposed: 5.8 ms instead of 4.1 ms for the two contractions.
 
-// the CTA-pair kernel needs BN/2 to be a multiple of 8 rows and an even number of padded m-tiles
+// Tile widths of 128 columns and more run on the CTA-pair kernel (BN/2 weight rows per CTA, a multiple of 8), 64 on the
+// single-CTA kernel.  A pair owns two consecutive m-tiles, so the A image of a pair launch must cover an even number of
+// m-tiles even when m_tiles is odd: every caller pads its activation images to a multiple of 2 * BM rows.
 template <int BN>
 int launch_gemm(const GemmArgs& g, cudaStream_t st) {
-  const bool pair_kernel = g.pair_ok && BN >= 128 && (g.f8 || gemm_pair_mode());
-  AZG_REQUIRE(!(g.kbn || g.kb0 || g.acc_in || g.no_bias || g.side_acc) || (g.x3 && pair_kernel && g.kb0 >= 0 && g.kb0 + g.kbn <= g.KB),
-              "tcgen05 GEMM: K-split launches run on the CTA-pair kernel of the split precisions only");
-  AZG_REQUIRE(g.ksplit <= 1 || (g.x3 && pair_kernel && g.kpart && !g.kbn && !g.acc_in && g.KB >= g.ksplit),
-              "tcgen05 GEMM: the in-kernel K-split runs on the CTA-pair kernel of the split precisions only");
-  if (g.f8) {
-    if constexpr (BN >= 128 && BN <= 224) {
-      AZG_REQUIRE(g.pair_ok && g.x3, "tcgen05 GEMM: the fp16+FP8 split runs on the CTA-pair kernel only");
-      return launch_gemm_impl<BN, true>(g, st);
-    } else {
-      azg_set_error("tcgen05 GEMM: the fp16+FP8 split needs a tile width of 128..224 columns");
-      return AZG_ERR_INVALID;
-    }
+  const bool ksplit_launch = g.kbn || g.kb0 || g.acc_in || g.no_bias || g.side_acc;
+  if constexpr (BN >= 128) {
+    AZG_REQUIRE(!ksplit_launch || (g.x3 && g.kb0 >= 0 && g.kb0 + g.kbn <= g.KB),
+                "tcgen05 GEMM: K-split launches run on the split precisions only");
+    AZG_REQUIRE(g.ksplit <= 1 || (g.x3 && g.kpart && !g.kbn && !g.acc_in && g.KB >= g.ksplit),
+                "tcgen05 GEMM: the in-kernel K-split runs on the split precisions only");
+    AZG_REQUIRE(!g.f8 || (BN <= 224 && g.x3), "tcgen05 GEMM: the fp16+FP8 split needs a tile width of 128..224 columns");
+    return launch_gemm_impl<BN, true>(g, st);
+  } else {
+    AZG_REQUIRE(!ksplit_launch && g.ksplit <= 1 && !g.f8 && !g.side_hi,
+                "tcgen05 GEMM: the K-split, the fp16+FP8 split and the side tile run on the CTA-pair kernel (tile width >= 128)");
+    return launch_gemm_impl<BN, false>(g, st);
   }
-  if (gemm_pair_mode() && g.pair_ok && BN >= 128) return launch_gemm_impl<BN, true>(g, st);
-  return launch_gemm_impl<BN, false>(g, st);
 }
 
 // partial head-sum slots per n-tile (one per epilogue group)
@@ -779,7 +748,6 @@ int run_gemm(int BN, const GemmArgs& g, cudaStream_t st) {
     case 160: return launch_gemm<160>(g, st);
     case 128: return launch_gemm<128>(g, st);
     case 64: return launch_gemm<64>(g, st);
-    case 32: return launch_gemm<32>(g, st);
   }
   azg_set_error("tcgen05 GEMM: no tile width for this feature size");
   return AZG_ERR_INVALID;
@@ -796,62 +764,8 @@ int to_image(const float* src, int64_t rows, int64_t rows_padded, int K, int R, 
 
 // ---- Connect4 trunk on the tensor cores ------------------------------------------------------
 // conv2 (32 -> 64 channels, 3x3, pad 1) as an implicit GEMM:  rows m = (board b, cell p),
-// K = (tap, cin) = 9*32 = 288 (padded to 320 = 5 k-blocks), N = 64 output channels.  This kernel
-// evaluates conv1 + ReLU on the fly from the packed position (K1 encode fused in) and writes the
-// im2col operand directly as tile images (hi/lo bf16), 1280 B per row.
+// K = (tap, cin) = 9*32 = 288 (padded to 320 = 5 k-blocks), N = 64 output channels.
 constexpr int C2_K = 320, C2_KB = C2_K / BK;
-
-__global__ void __launch_bounds__(256) c4_im2col_kernel(const uint64_t* __restrict__ states, int n, int64_t B,
-                                                        const float* __restrict__ w1, const float* __restrict__ b1,
-                                                        uint8_t* __restrict__ a_hi, uint8_t* __restrict__ a_lo) {
-  __shared__ float planes[100];            // (n+2)^2 board with a zero border
-  __shared__ __align__(16) float a1s[100 * 32];  // relu(conv1) per padded cell, 32 channels each, zero border
-  __shared__ float w1s[32 * 9], b1s[32];
-  const int np = n + 2, nn = n * n;
-  for (int i = threadIdx.x; i < 100 * 32; i += blockDim.x) a1s[i] = 0.0f;
-  for (int i = threadIdx.x; i < 32 * 9; i += blockDim.x) w1s[i] = w1[i];
-  if (threadIdx.x < 32) b1s[threadIdx.x] = b1[threadIdx.x];
-  for (int64_t b = blockIdx.x; b < B; b += gridDim.x) {
-    __syncthreads();
-    const uint64_t mine = states[2 * b], theirs = states[2 * b + 1];
-    for (int i = threadIdx.x; i < np * np; i += blockDim.x) {
-      const int x = i / np - 1, y = i % np - 1;
-      float v = 0.0f;
-      if (x >= 0 && x < n && y >= 0 && y < n) {
-        const int c = x * n + y;
-        v = (float)((int)((mine >> c) & 1ull) - (int)((theirs >> c) & 1ull));
-      }
-      planes[i] = v;
-    }
-    __syncthreads();
-    for (int o = threadIdx.x; o < 32 * nn; o += blockDim.x) {  // conv1 + ReLU, Connect4Net.py:45
-      const int ci = o & 31, pc = o >> 5, x = pc / n, y = pc % n;
-      float acc = b1s[ci];
-#pragma unroll
-      for (int kx = 0; kx < 3; ++kx)
-#pragma unroll
-        for (int ky = 0; ky < 3; ++ky) acc = fmaf(planes[(x + kx) * np + y + ky], w1s[ci * 9 + kx * 3 + ky], acc);
-      a1s[((x + 1) * np + y + 1) * 32 + ci] = fmaxf(acc, 0.0f);
-    }
-    __syncthreads();
-    for (int task = threadIdx.x; task < nn * (C2_K / 8); task += blockDim.x) {
-      const int pc = task / (C2_K / 8), c = task % (C2_K / 8);
-      float x8[8];
-      if (c < 36) {
-        const int tap = c >> 2, ci0 = (c & 3) * 8, kx = tap / 3, ky = tap % 3, x = pc / n, y = pc % n;
-        const float4* src = reinterpret_cast<const float4*>(a1s + ((x + kx) * np + y + ky) * 32 + ci0);
-        const float4 u = src[0], w = src[1];
-        x8[0] = u.x; x8[1] = u.y; x8[2] = u.z; x8[3] = u.w; x8[4] = w.x; x8[5] = w.y; x8[6] = w.z; x8[7] = w.w;
-      } else {
-#pragma unroll
-        for (int e = 0; e < 8; ++e) x8[e] = 0.0f;
-      }
-      const int64_t m = b * nn + pc;
-      const size_t off = ((size_t)(m >> 7) * C2_KB + (c >> 3)) * A_STAGE_BYTES + image_offset((int)(m & 127), (c & 7) * 8);
-      split_store(x8, a_hi, a_lo, off);
-    }
-  }
-}
 
 // conv2 weights [64,32,3,3] -> [64 x 320] image, k = tap*32 + cin (zero padded)
 __global__ void conv2_weight_image_kernel(const float* __restrict__ w2, uint8_t* __restrict__ hi, uint8_t* __restrict__ lo) {
@@ -892,88 +806,6 @@ __global__ void __launch_bounds__(256) permuted_weight_image_kernel(const float*
   }
   const size_t off = ((size_t)(row / R) * KB + (c >> 3)) * ((size_t)R * 128) + image_offset(row % R, (c & 7) * 8);
   split_store(x8, hi, lo, off);
-}
-
-// head weights (policy rows then the value row) permuted to the feature image's order, fp32
-__global__ void permute_heads_kernel(const float* __restrict__ wp, const float* __restrict__ wv, int A, int F, int nn,
-                                     float* __restrict__ out) {
-  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (idx >= (int64_t)(A + 1) * F) return;
-  const int row = (int)(idx / F), kp = (int)(idx % F), pc = kp >> 6, co = kp & 63;
-  const float* src = row < A ? wp + (size_t)row * F : wv;
-  out[idx] = src[co * nn + pc];
-}
-
-__device__ __forceinline__ float warp_sum(float v) {
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-  return v;
-}
-
-__device__ __forceinline__ void unpack_bf16x8(const uint4 u, float* f) {
-  const uint32_t w[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-  for (int e = 0; e < 4; ++e) {
-    f[2 * e] = __uint_as_float(w[e] << 16);
-    f[2 * e + 1] = __uint_as_float(w[e] & 0xffff0000u);
-  }
-}
-
-// standard heads (predict, Connect4Net.py:55-60) straight from the feature image: one warp per position
-template <int MAXA>
-__global__ void __launch_bounds__(256) heads_image_kernel(const uint8_t* __restrict__ f_hi, const uint8_t* __restrict__ f_lo,
-                                                          int KB, const float* __restrict__ wperm,
-                                                          const float* __restrict__ bp, const float* __restrict__ bv, int A,
-                                                          int64_t B, float* __restrict__ pi, float* __restrict__ v) {
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int F = KB * BK;
-  for (int64_t row = (int64_t)blockIdx.x * 8 + warp; row < B; row += (int64_t)gridDim.x * 8) {
-    const size_t tile0 = (size_t)(row >> 7) * KB * A_STAGE_BYTES;
-    const int r = (int)(row & 127);
-    float acc[MAXA + 1];
-#pragma unroll
-    for (int a = 0; a <= MAXA; ++a) acc[a] = 0.0f;
-    for (int q = lane; q < KB * 8; q += 32) {
-      const int kb = q >> 3, j = q & 7;
-      const size_t off = tile0 + (size_t)kb * A_STAGE_BYTES + image_offset(r, j * 8);
-      float f[8], l[8];
-      unpack_bf16x8(*reinterpret_cast<const uint4*>(f_hi + off), f);
-      if (f_lo) {
-        unpack_bf16x8(*reinterpret_cast<const uint4*>(f_lo + off), l);
-#pragma unroll
-        for (int e = 0; e < 8; ++e) f[e] += l[e];
-      }
-      const int kp = kb * BK + j * 8;
-#pragma unroll
-      for (int a = 0; a <= MAXA; ++a) {
-        if (a <= A) {  // rows 0..A-1 policy, row A value
-          const float4 w0 = __ldg(reinterpret_cast<const float4*>(wperm + (size_t)a * F + kp));
-          const float4 w1 = __ldg(reinterpret_cast<const float4*>(wperm + (size_t)a * F + kp + 4));
-          acc[a] = fmaf(f[0], w0.x, fmaf(f[1], w0.y, fmaf(f[2], w0.z, fmaf(f[3], w0.w, acc[a]))));
-          acc[a] = fmaf(f[4], w1.x, fmaf(f[5], w1.y, fmaf(f[6], w1.z, fmaf(f[7], w1.w, acc[a]))));
-        }
-      }
-    }
-    float logit[MAXA + 1];
-#pragma unroll
-    for (int a = 0; a <= MAXA; ++a) logit[a] = warp_sum(acc[a]);
-    float m = -INFINITY;
-#pragma unroll
-    for (int a = 0; a < MAXA; ++a)
-      if (a < A) { logit[a] += __ldg(bp + a); m = fmaxf(m, logit[a]); }
-    float sum = 0.0f;
-#pragma unroll
-    for (int a = 0; a < MAXA; ++a)
-      if (a < A) sum += expf(logit[a] - m);
-    const float lse = logf(sum);
-    float vraw = 0.0f;
-#pragma unroll
-    for (int a = 0; a <= MAXA; ++a) {
-      if (a < A && lane == a) pi[row * A + a] = expf((logit[a] - m) - lse);
-      if (a == A) vraw = logit[a];
-    }
-    if (lane == 0) v[row] = tanhf(vraw + __ldg(bv));
-  }
 }
 
 // logits = fixed-order sum of the per-tile partial head sums + bias; then exp(log_softmax) and tanh
@@ -1065,7 +897,7 @@ __global__ void concat_heads_kernel(const float* __restrict__ wp, const float* _
   out[idx] = row < A ? wp[(size_t)row * F + k] : (row == A ? wv[k] : 0.0f);
 }
 
-// std heads from the [B,32] logits block produced by the skinny tensor-core GEMM (bias already added)
+// std heads from the [B,32] logits block produced by GEMM-1's side tile (bias already added)
 __global__ void heads32_finalize_kernel(const float* __restrict__ lg, int A, int64_t B, const int32_t* __restrict__ dyn_rows,
                                         float* __restrict__ pi, float* __restrict__ v) {
   const int64_t row = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -1080,46 +912,34 @@ __global__ void heads32_finalize_kernel(const float* __restrict__ lg, int A, int
   v[row] = tanhf(x[A]);
 }
 
-// ---- fused trunk: encode + conv1 + im2col in shared memory -> tcgen05 conv2 --------------------
-// One persistent CTA per SM, 16 warps.  A tile is G = 128 / n^2 whole boards (G*n^2 <= 128 GEMM rows).
-//   warps 0-7   builders, two threads per tile row (r = tid & 127, half = tid >> 7):
-//               (1) K1 encode + conv1 operand: the 3x3 neighbourhood of the row's cell, read straight from the packed
-//                   position (bits -> bf16 {-1, 0, +1}), written three times along K into a ring stage ("C1 slot");
-//                   conv1 itself runs on the tensor core against [w_hi | w_mid | w_lo] (three bf16 terms = the full
-//                   fp32 weight, the {-1,0,1} operand is exact, fp32 accumulation): 3 MMAs of 128 x 32 x 16 per tile;
-//               (2) conv1 "epilogue": TMEM -> +bias, ReLU -> bf16 hi/lo into the padded cell plane in smem (64-byte
-//                   cells, zero border) -- each thread converts 16 channels of its own cell;
-//               (3) per k-block copy the 3x3 patches into the SWIZZLE_128B operand stage (pure 16-byte smem->smem
-//                   moves, a quarter-warp per tile row), fence.proxy.async, arrive on the stage's mbarrier.
-//               The C1 slot of tile i+1 is queued between k-blocks 2 and 3 of tile i, so its MMAs have long completed
-//               when the builders come back for (2).
-//   warp 8      MMA issuer (one thread): conv2 M=128 x N=64 x K=16 (weight images resident in smem), conv1 as above
-//   warp 9      TMEM allocation, barrier init, one-time bulk copy of the conv2 weight images
-//   warps 12-15 epilogue: TMEM -> +bias, ReLU -> feature image (the A operand of GEMM-1)
-// The im2col matrix never exists in HBM (the split version moved 2 x 4.1 GB per 65,536 positions).
-// History of conv1: FFMA with lanes = channels and broadcast LDS of the planes took 42 % of the builders' time
-// (ncu source view of the round-1 v6 capture, since pruned: 18 LDS per two cells queued behind the tensor core's own
-// shared-memory reads); on the tensor core it is 3 MMAs and one tcgen05.ld per thread.
-constexpr int TR_THREADS = 512;
-constexpr int TR_CELL_STRIDE = 64;   // bytes per padded cell: 32 channels x bf16, no pad (see the patch copies)
-constexpr int TR_MAX_CELLS = 288;    // max over n of G * (n+2)^2
+// ---- fused trunk: encode + conv1 + conv2 in one kernel on the tensor cores ----------------------------------------------
+// One persistent CTA per SM, 20 warps.  conv2 is an implicit GEMM over SHIFTED operand descriptors:
+//   * relu(conv1) of a tile's boards is stored in a padded plane of 128-byte cells [32 ch hi (64 B) | 32 ch lo (64 B)],
+//     SWIZZLE_128B by the cell index, raster pitch n+1: the right border of a board row IS the left border of the next row
+//     and the bottom border row of a board IS the top border row of the next board, so board b's cell (x, y) sits at plane
+//     cell b (n+1)^2 + (x+1)(n+1) + (y+1);
+//   * GEMM row r = b (n+1)^2 + x (n+1) + y (the position of tap (0,0)); tap (kx, ky) of EVERY row is then plane cell
+//     r + kx (n+1) + ky: the A operand of a tap is the same 128 rows at a different START ADDRESS (any multiple of 128 B:
+//     the tensor core applies the 128-byte swizzle to absolute shared-memory address bits, so a plane written with
+//     chunk ^ (cell & 7) reads back correctly from every start; measured on B200 -- with the descriptor's base-offset
+//     field set to the start's phase the results are WRONG, with the field left 0 they equal an explicit im2col operand
+//     bit for bit), K-advance inside the 128-byte cell selects hi / lo and the 16-channel half.
+//     18 K = 16 steps (9 taps x 2) against the [64 x 320] conv2 weight image, no patch copies, no padded k-block.
+//     (Copying the nine patches of every cell into operand stages instead cost 320 KB of shared-memory -> shared-memory
+//     traffic per 128-row tile on top of the tensor core's own 280 KB of operand reads: 1.04-1.12 instead of 0.61-0.71 ms
+//     per step of 65,536 positions, profiles/r01_trunk_fused_v8.txt and r02_trunk_fused2.txt.)
+// Rows between boards compute garbage from border / neighbouring cells and are dropped by the epilogue (n = 7: 2 boards per
+// tile, rows 0-54 and 64-118).
+// conv1 runs on the tensor core too: the builder warps (two threads per tile row) encode the 3x3 neighbourhood of the row's
+// cell straight from the packed position (bits -> bf16 {-1, 0, +1}), written three times along K into a conv1 operand stage,
+// against [w_hi | w_mid | w_lo] (three bf16 terms = the full fp32 weight, the {-1,0,1} operand is exact, fp32 accumulation):
+// 3 MMAs of 128 x 32 x 16 per tile; the builders read the result back from TMEM (+bias, ReLU, hi/lo split into the plane).
+// (As FFMA with lanes = channels and broadcast LDS of the planes, conv1 took 42 % of the builders' time: 18 LDS per two
+// cells queued behind the tensor core's own shared-memory reads; on the tensor core it is 3 MMAs and one tcgen05.ld per
+// thread.)  Planes, conv1 operand stages and conv1 TMEM regions are double-buffered so that tile i+1's conv1 and plane
+// write-back run under tile i's 36 conv2 MMAs.
 constexpr int TR_W_BYTES = C2_KB * 64 * 128;  // conv2 weight image [64 x 320] bf16 = 40 KB
 constexpr int TR_W1_BYTES = 32 * 128;         // conv1 weight image [32 x 64] bf16: cols 0-8 hi, 16-24 mid, 32-40 lo
-constexpr int TR_C1_AFTER_KB = 2;             // the next tile's C1 slot follows this k-block in the ring
-
-template <bool X3>
-struct TrunkSmem {
-  static constexpr int STAGES = X3 ? 3 : 4;
-  static constexpr int STAGE_BYTES = (X3 ? 2 : 1) * A_STAGE_BYTES;
-  static constexpr int W_OFF = 0;
-  static constexpr int W1_OFF = (X3 ? 2 : 1) * TR_W_BYTES;
-  static constexpr int A1_OFF = W1_OFF + TR_W1_BYTES;
-  static constexpr int A1_BYTES = ((TR_MAX_CELLS * TR_CELL_STRIDE + 1023) / 1024) * 1024;
-  static constexpr int STAGE_OFF = A1_OFF + (X3 ? 2 : 1) * A1_BYTES;
-  static constexpr int MISC_OFF = STAGE_OFF + STAGES * STAGE_BYTES;
-  static constexpr int TOTAL = MISC_OFF + 1024 + 1024;  // barriers + alignment slack
-};
-
 struct TrunkArgs {
   const uint64_t* states;
   const float *w1, *b1, *b2;   // conv1 weights/bias, conv2 bias
@@ -1131,372 +951,6 @@ struct TrunkArgs {
   int out_f8;               // feature image in the AZG_PREC_F16F8 activation format (the convolutions stay bf16x3)
 };
 
-template <bool X3>
-__global__ void __launch_bounds__(TR_THREADS, 1) c4_trunk_tc_kernel(TrunkArgs t) {
-  using S = TrunkSmem<X3>;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);  // stays a shared-space pointer (LDS/STS)
-  uint8_t* w_s = smem + S::W_OFF;
-  uint8_t* w1img = smem + S::W1_OFF;
-  uint8_t* a1hi = smem + S::A1_OFF;
-  uint8_t* a1lo = a1hi + S::A1_BYTES;
-  uint8_t* stages = smem + S::STAGE_OFF;
-  uint64_t* full = (uint64_t*)(smem + S::MISC_OFF);
-  uint64_t* empty = full + S::STAGES;
-  uint64_t* tfull = empty + S::STAGES;
-  uint64_t* tempty = tfull + 2;
-  uint64_t* wbar = tempty + 2;
-  uint64_t* c1done = wbar + 1;
-  uint32_t* tmem_slot = (uint32_t*)(c1done + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n = t.n, nn = n * n, np = n + 2, cells = np * np;
-  const int G = 128 / nn;  // boards per tile
-  if (t.dyn_rows && *t.dyn_rows < t.B) t.B = *t.dyn_rows;
-  const int64_t tiles = (t.B + G - 1) / G;
-  constexpr int BN = 64;
-  // bf16x3: A_hi meets [W_hi ; W_lo] in ONE N = 128 MMA (columns 0-63 = hi x hi, 64-127 = hi x lo), A_lo x W_hi
-  // accumulates into columns 0-63, and the epilogue adds the two halves: 14 KB instead of 18 KB of operand reads per
-  // K = 16 step (an N = 64 MMA needs 6 KB per 32 tensor cycles, more than the 128 B/clk shared memory delivers)
-  constexpr int ACC_COLS = X3 ? 128 : 64;  // TMEM columns per accumulator stage
-  constexpr uint32_t TMEM_COLS = X3 ? 512 : 256;
-  constexpr uint32_t C1_COL = 2 * ACC_COLS;  // conv1 result columns
-
-  // one-time setup
-  for (int i = threadIdx.x; i < (X3 ? 2 : 1) * S::A1_BYTES / 16; i += blockDim.x) reinterpret_cast<uint4*>(a1hi)[i] = make_uint4(0, 0, 0, 0);
-  for (int i = threadIdx.x; i < S::STAGES * S::STAGE_BYTES / 16; i += blockDim.x) reinterpret_cast<uint4*>(stages)[i] = make_uint4(0, 0, 0, 0);
-  for (int i = threadIdx.x; i < 32 * 64; i += blockDim.x) {  // conv1 weights as three bf16 terms along K (Connect4Net.py:32)
-    const int ch = i >> 6, col = i & 63, term = col >> 4, k = col & 15;
-    float v = 0.0f;
-    if (term < 3 && k < 9) {
-      const float w = t.w1[ch * 9 + k];
-      const float hi = __bfloat162float(__float2bfloat16_rn(w));
-      const float mid = __bfloat162float(__float2bfloat16_rn(w - hi));
-      v = term == 0 ? hi : term == 1 ? mid : (w - hi) - mid;
-    }
-    *reinterpret_cast<__nv_bfloat16*>(w1img + image_offset(ch, col)) = __float2bfloat16_rn(v);
-  }
-  if (warp == 9 && lane == 0) {
-    for (int s = 0; s < S::STAGES; ++s) {
-      mbar_init(&full[s], 256);
-      mbar_init(&empty[s], 1);
-    }
-    for (int a = 0; a < 2; ++a) {
-      mbar_init(&tfull[a], 1);
-      mbar_init(&tempty[a], 128);
-    }
-    mbar_init(wbar, 1);
-    mbar_init(c1done, 1);
-    fence_barrier_init();
-  }
-  if (warp == 9) tmem_alloc(tmem_slot, TMEM_COLS);
-  fence_async_smem();  // the zero-filled stages and the conv1 weight image are read by the tensor core (async proxy)
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 9) {
-    if (lane == 0) {  // conv2 weight images -> smem, once
-      mbar_expect_tx(wbar, (X3 ? 2 : 1) * TR_W_BYTES);
-      if (X3) {  // per k-block [hi 8 KB | lo 8 KB]: one 128-row B operand
-        for (int kb = 0; kb < C2_KB; ++kb) {
-          bulk_g2s(w_s + kb * 16384, t.w_hi + kb * 8192, 8192, wbar);
-          bulk_g2s(w_s + kb * 16384 + 8192, t.w_lo + kb * 8192, 8192, wbar);
-        }
-      } else {
-        bulk_g2s(w_s, t.w_hi, TR_W_BYTES, wbar);
-      }
-    }
-  } else if (warp < 8) {
-    // ============ builders: 8 warps, two threads per tile row ============
-    const int r = threadIdx.x & 127, half = threadIdx.x >> 7;  // tile row, half (16 conv1 channels / 3 operand chunks)
-    const int bl = r / nn, pc = r - bl * nn, x = pc / n, y = pc - x * n;
-    const bool row_valid = bl < G;
-    const int cell0 = bl * cells + x * np + y;  // padded cell of tap (0,0); tap (kx,ky) adds kx*np + ky
-    // taps of this row's cell that lie on the board (bit k = tap kx*3+ky), fixed for the whole kernel
-    uint32_t tap_ok = 0;
-#pragma unroll
-    for (int k = 0; k < 9; ++k) {
-      const int xx = x + k / 3 - 1, yy = y + k % 3 - 1;
-      if (row_valid && xx >= 0 && xx < n && yy >= 0 && yy < n) tap_ok |= 1u << k;
-    }
-    // patch-copy mapping: lane & 7 = chunk of the k-block, rows grow0 + 32 i
-    const int gj = threadIdx.x & 7, grow0 = threadIdx.x >> 3;
-    int gcell[4];
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-      const int rr_ = grow0 + 32 * i, b_ = rr_ / nn, p_ = rr_ - b_ * nn, x_ = p_ / n;
-      gcell[i] = b_ < G ? b_ * cells + x_ * np + (p_ - x_ * n) : -1;
-    }
-    float bias16[16];
-#pragma unroll
-    for (int j = 0; j < 16; ++j) bias16[j] = __ldg(t.b1 + half * 16 + j);
-    const uint32_t c1_taddr = tmem_base + ((uint32_t)((warp & 3) * 32) << 16) + C1_COL + (uint32_t)(half * 16);
-    int stage = 0;
-    uint32_t phase = 0, c1_phase = 0;
-    // the packed positions are fetched one tile ahead of their use (global latency off the critical path)
-    uint64_t nm = 0, nt = 0;
-    auto fetch = [&](int64_t tile) {
-      nm = nt = 0;
-      const int64_t b = tile * G + bl;
-      if (row_valid && tile < tiles && b < t.B) { nm = t.states[2 * b]; nt = t.states[2 * b + 1]; }
-    };
-    // K1 encode + conv1 operand of the tile whose position is in (nm, nt): 16 bf16 = taps 0..8 and zeros, the same
-    // 32 bytes at K = 0, 16 and 32 (one copy per weight term); this thread writes three of the six 16-byte chunks
-    auto c1_slot = [&]() {
-      mbar_wait(&empty[stage], phase ^ 1);
-      uint8_t* sa = stages + stage * S::STAGE_BYTES;
-      uint32_t pk[5];
-#pragma unroll
-      for (int k = 0; k < 9; ++k) {
-        const int sh = (pc + (k / 3 - 1) * n + (k % 3 - 1)) & 63;
-        const uint32_t ok = (tap_ok >> k) & 1u;
-        const uint32_t m = (uint32_t)(nm >> sh) & ok, o = (uint32_t)(nt >> sh) & ok;
-        const uint32_t v = (m ? 0x3F80u : 0u) | (o ? 0xBF80u : 0u);  // bf16 +1 / -1
-        if (k & 1) pk[k >> 1] |= v << 16;
-        else pk[k >> 1] = v;
-      }
-      const uint4 c_even = make_uint4(pk[0], pk[1], pk[2], pk[3]), c_odd = make_uint4(pk[4], 0, 0, 0);
-#pragma unroll
-      for (int j = 0; j < 3; ++j) {
-        const int c = half * 3 + j;  // chunk 0..5 of the row: even chunks = taps 0-7, odd chunks = tap 8
-        *reinterpret_cast<uint4*>(sa + image_offset(r, c * 8)) = (c & 1) ? c_odd : c_even;
-      }
-      fence_async_smem();
-      mbar_arrive(&full[stage]);
-      if (++stage == S::STAGES) {
-        stage = 0;
-        phase ^= 1;
-      }
-    };
-    fetch(blockIdx.x);
-    if ((int64_t)blockIdx.x < tiles) c1_slot();
-    fetch((int64_t)blockIdx.x + gridDim.x);
-    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-      const bool has_next = tile + gridDim.x < tiles;
-      // relu(conv1 + bias) of this row's cell, 16 channels: TMEM -> bf16 hi/lo in the padded plane (Connect4Net.py:45)
-      mbar_wait(c1done, c1_phase);
-      c1_phase ^= 1;
-      tc_fence_after();
-      uint32_t rr[16];
-      tmem_ld16(c1_taddr, rr);
-      tmem_ld_wait();
-      tc_fence_before();
-      if (row_valid) {
-        float v[16];
-#pragma unroll
-        for (int j = 0; j < 16; ++j) v[j] = fmaxf(__uint_as_float(rr[j]) + bias16[j], 0.0f);
-        const uint32_t off = (uint32_t)(cell0 + np + 1) * TR_CELL_STRIDE + half * 32;
-        split_store(v, a1hi, X3 ? a1lo : nullptr, off);
-        split_store(v + 8, a1hi, X3 ? a1lo : nullptr, off + 16);
-      }
-      named_bar(2, 256);  // conv1 output complete
-      for (int kb = 0; kb < C2_KB; ++kb) {
-        // Patch copies: the 8 lanes of a quarter-warp move the 8 chunks (two taps x 64 B) of ONE tile row, so a
-        // 128-bit shared load touches two 64-byte cells whose offsets differ by an odd number of cells (tap +1, or
-        // n cells across a kernel row for odd n): distinct bank groups.  (One row per lane with an 80-byte cell
-        // stride conflicted 2-way whenever the 8 rows of a quarter-warp crossed a board-row end: +48 % wavefronts.)
-        // All loads of the k-block are issued before the wait for a free stage and before any store (the compiler
-        // cannot reorder shared loads over shared stores itself: four dependent round trips became one).
-        const int c = kb * 8 + gj;  // 16-byte chunk of the K = (tap, cin) axis
-        const bool chunk_live = c < 36;
-        const int tap = c >> 2, kx = tap / 3, ky = tap - kx * 3;
-        const uint32_t toff = (uint32_t)((kx * np + ky) * TR_CELL_STRIDE + (c & 3) * 16);
-        uint4 vh[4], vl[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          vh[i] = make_uint4(0, 0, 0, 0);
-          vl[i] = make_uint4(0, 0, 0, 0);
-          if (gcell[i] >= 0 && chunk_live) {
-            const uint32_t src = (uint32_t)gcell[i] * TR_CELL_STRIDE + toff;
-            vh[i] = *reinterpret_cast<const uint4*>(a1hi + src);
-            if (X3) vl[i] = *reinterpret_cast<const uint4*>(a1lo + src);
-          }
-        }
-        mbar_wait(&empty[stage], phase ^ 1);
-        uint8_t* sa = stages + stage * S::STAGE_BYTES;
-#pragma unroll
-        for (int i = 0; i < 4; ++i) {
-          if (gcell[i] >= 0) {
-            const uint32_t dst = image_offset(grow0 + 32 * i, gj * 8);
-            *reinterpret_cast<uint4*>(sa + dst) = vh[i];
-            if (X3) *reinterpret_cast<uint4*>(sa + A_STAGE_BYTES + dst) = vl[i];
-          }
-        }
-        fence_async_smem();  // generic-proxy writes -> visible to the tensor core's async-proxy reads
-        mbar_arrive(&full[stage]);
-        if (++stage == S::STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
-        if (kb == TR_C1_AFTER_KB && has_next) {  // conv1 operand of the next tile, then fetch the one after
-          c1_slot();
-          fetch(tile + 2 * (int64_t)gridDim.x);
-        }
-      }
-      named_bar(1, 256);  // every builder is done reading this tile's conv1 output
-    }
-  } else if (warp == 8) {
-    // ======================= MMA issuer =======================
-    if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(BM, BN);
-      constexpr uint32_t idesc_c1 = make_idesc(BM, 32);
-      constexpr uint32_t idesc_cat = make_idesc(BM, 2 * BN);
-      mbar_wait(wbar, 0);
-      const uint32_t w_addr = smem_u32(w_s);
-      const uint64_t b_c1 = make_smem_desc(smem_u32(w1img));
-      int stage = 0, acc = 0;
-      uint32_t phase = 0, acc_phase = 0;
-      auto c1_slot = [&]() {  // conv1 of one tile: [A | A | A] x [w_hi | w_mid | w_lo]^T -> TMEM columns C1_COL..+31
-        mbar_wait(&full[stage], phase);
-        tc_fence_after();
-        const uint64_t a_c1 = make_smem_desc(smem_u32(stages + stage * S::STAGE_BYTES));
-#pragma unroll
-        for (int k = 0; k < 3; ++k) umma_bf16(tmem_base + C1_COL, a_c1 + 2 * k, b_c1 + 2 * k, idesc_c1, k != 0);
-        umma_commit(&empty[stage]);
-        umma_commit(c1done);
-        if (++stage == S::STAGES) {
-          stage = 0;
-          phase ^= 1;
-        }
-      };
-      if ((int64_t)blockIdx.x < tiles) c1_slot();
-      for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-        const bool has_next = tile + gridDim.x < tiles;
-        mbar_wait(&tempty[acc], acc_phase ^ 1);
-        tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(acc * ACC_COLS);
-        for (int kb = 0; kb < C2_KB; ++kb) {
-          mbar_wait(&full[stage], phase);
-          tc_fence_after();
-          const uint32_t sa = smem_u32(stages + stage * S::STAGE_BYTES);
-          const uint64_t a_hi = make_smem_desc(sa), a_lo = make_smem_desc(sa + A_STAGE_BYTES);
-          const uint64_t b_w = make_smem_desc(w_addr + kb * (X3 ? 2 : 1) * (64 * 128));  // X3: rows 0-63 hi, 64-127 lo
-          if (X3) {
-#pragma unroll
-            for (int k = 0; k < BK / 16; ++k) umma_bf16(d_tmem, a_hi + 2 * k, b_w + 2 * k, idesc_cat, (kb | k) != 0);
-#pragma unroll
-            for (int k = 0; k < BK / 16; ++k) umma_bf16(d_tmem, a_lo + 2 * k, b_w + 2 * k, idesc, 1);
-          } else {
-#pragma unroll
-            for (int k = 0; k < BK / 16; ++k) umma_bf16(d_tmem, a_hi + 2 * k, b_w + 2 * k, idesc, (kb | k) != 0);
-          }
-          umma_commit(&empty[stage]);
-          if (++stage == S::STAGES) {
-            stage = 0;
-            phase ^= 1;
-          }
-          if (kb == TR_C1_AFTER_KB && has_next) c1_slot();
-        }
-        umma_commit(&tfull[acc]);
-        if (++acc == 2) {
-          acc = 0;
-          acc_phase ^= 1;
-        }
-      }
-    }
-  } else if (warp >= 12) {
-    // ======================= epilogue =======================
-    const int q = warp & 3, r = q * 32 + lane;
-    const int bl = r / nn, pc = r - bl * nn;
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
-      const int64_t b = tile * G + bl;
-      const bool valid = bl < G && b < t.B;
-      mbar_wait(&tfull[acc], acc_phase);
-      tc_fence_after();
-      const uint32_t taddr = tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(acc * ACC_COLS);
-      const size_t tbase = ((size_t)(b >> 7) * nn + pc) * A_STAGE_BYTES;
-      const int rb = (int)(b & 127);
-#pragma unroll 1
-      for (int c0 = 0; c0 < BN; c0 += 16) {
-        uint32_t rr[16], r2[16];
-        tmem_ld16(taddr + (uint32_t)c0, rr);
-        if (X3) tmem_ld16(taddr + (uint32_t)(BN + c0), r2);  // the hi x lo half
-        tmem_ld_wait();
-        if (valid && X3 && t.out_f8) {  // fp16 image + FP8 correction rows, one 16-byte chunk of each half per 16 channels
-          float x16[16];
-#pragma unroll
-          for (int e = 0; e < 16; ++e)
-            x16[e] = fmaxf(__uint_as_float(rr[e]) + __uint_as_float(r2[e]) + __ldg(t.b2 + c0 + e), 0.0f);
-          const float s_main = (float)(1 << F8_A_SCALE), s_lo = (float)(1 << (F8_A_SCALE + F8_LO_SHIFT));
-          uint4 h0, h1;
-          uint2 m0, m1, l0, l1;
-          split8_f16f8(x16, s_main, s_lo, h0, m0, l0);
-          split8_f16f8(x16 + 8, s_main, s_lo, h1, m1, l1);
-          *reinterpret_cast<uint4*>(t.f_hi + tbase + image_offset(rb, c0)) = h0;
-          *reinterpret_cast<uint4*>(t.f_hi + tbase + image_offset(rb, c0 + 8)) = h1;
-          *reinterpret_cast<uint4*>(t.f_lo + tbase + image_offset_bytes(rb, c0)) = make_uint4(m0.x, m0.y, m1.x, m1.y);
-          *reinterpret_cast<uint4*>(t.f_lo + tbase + image_offset_bytes(rb, 64 + c0)) = make_uint4(l0.x, l0.y, l1.x, l1.y);
-        } else if (valid) {
-#pragma unroll
-          for (int c = 0; c < 2; ++c) {
-            float x8[8];
-#pragma unroll
-            for (int e = 0; e < 8; ++e) {
-              float d = __uint_as_float(rr[c * 8 + e]);
-              if (X3) d += __uint_as_float(r2[c * 8 + e]);
-              x8[e] = fmaxf(d + __ldg(t.b2 + c0 + c * 8 + e), 0.0f);
-            }
-            split_store(x8, t.f_hi, X3 ? t.f_lo : nullptr, tbase + image_offset(rb, c0 + c * 8));
-          }
-        }
-      }
-      tc_fence_before();
-      mbar_arrive(&tempty[acc]);
-      if (++acc == 2) {
-        acc = 0;
-        acc_phase ^= 1;
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 9) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, TMEM_COLS);
-  }
-}
-
-template <bool X3>
-int launch_trunk(const TrunkArgs& t, cudaStream_t st) {
-  static bool configured = false;
-  int dev = 0, sms = 0;
-  AZG_CUDA_CHECK(cudaGetDevice(&dev));
-  AZG_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  if (!configured) {
-    AZG_CUDA_CHECK(cudaFuncSetAttribute(c4_trunk_tc_kernel<X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, TrunkSmem<X3>::TOTAL));
-    configured = true;
-  }
-  const int G = 128 / (t.n * t.n);
-  const int64_t tiles = (t.B + G - 1) / G;
-  const int grid = (int)(tiles < sms ? tiles : sms);
-  c4_trunk_tc_kernel<X3><<<grid, TR_THREADS, TrunkSmem<X3>::TOTAL, st>>>(t);
-  AZG_LAUNCH_CHECK();
-  return AZG_OK;
-}
-
-// ---- fused trunk, second generation: conv2 as an implicit GEMM over SHIFTED operand descriptors --------------------------
-// The first fused trunk copies every relu(conv1) cell nine times (once per tap) from the padded plane into SWIZZLE_128B operand
-// stages: 320 KB of shared-memory -> shared-memory traffic per 128-row tile on top of the tensor core's own 280 KB of
-// operand reads, which is what bounds it (data pipe, tensor pipe 28 %).  Here the tensor core reads the padded plane itself:
-//   * the plane is stored as 128-byte cells [32 ch hi (64 B) | 32 ch lo (64 B)], SWIZZLE_128B by the cell index, raster
-//     pitch n+1: the right border of a board row IS the left border of the next row and the bottom border row of a board IS
-//     the top border row of the next board, so board b's cell (x, y) sits at plane cell b (n+1)^2 + (x+1)(n+1) + (y+1);
-//   * GEMM row r = b (n+1)^2 + x (n+1) + y (the position of tap (0,0)); tap (kx, ky) of EVERY row is then plane cell
-//     r + kx (n+1) + ky: the A operand of a tap is the same 128 rows at a different START ADDRESS (any multiple of 128 B:
-//     the tensor core applies the 128-byte swizzle to absolute shared-memory address bits, so a plane written with
-//     chunk ^ (cell & 7) reads back correctly from every start; measured on B200 -- with the descriptor's base-offset
-//     field set to the start's phase the results are WRONG, with the field left 0 they equal the first-generation trunk
-//     bit for bit), K-advance inside the 128-byte cell selects hi / lo and the 16-channel half.
-//     18 K = 16 steps (9 taps x 2), no patch copies, no padded k-block.
-// Rows between boards compute garbage from border / neighbouring cells and are dropped by the epilogue (n = 7: 2 boards per
-// tile, rows 0-54 and 64-118).  conv1 stays on the tensor core as before (operand built from the packed position by the
-// builder warps, result read back from TMEM, bias + ReLU, hi/lo split into the plane); planes, conv1 operand stages and
-// conv1 TMEM regions are double-buffered so that tile i+1's conv1 and plane write-back run under tile i's 36 conv2 MMAs.
 constexpr int T2_PLANE_CELLS = 152;                       // 128 rows + 2 (n+1) + 2 tap reach, n <= 8
 constexpr int T2_PLANE_BYTES = T2_PLANE_CELLS * 128;      // 19 KB, 1024-byte multiple
 
@@ -1513,14 +967,10 @@ struct Trunk2Smem {
 
 constexpr int T2_THREADS = 640;  // 8 builder warps, MMA, TMEM/barrier setup, 2 idle, 2 x 4 epilogue warps
 
-// PAIR (AZG_TRUNK=fused2pair, not the default): a cluster of two CTAs issues every tcgen05.mma ONCE for both CTAs' tiles
-// (cta_group::2, M = 256) and each CTA reads only its half of the weight operand.  Bit-identical to the single-CTA kernel and
-// measured at the same speed (0.655 vs 0.63-0.67 ms, profiles/r02_trunk_fused2.txt): the instruction count was not the bound.  Everything else stays per CTA (builders, planes, conv1 operand stages, epilogue); the peer CTA's MMA warp
-// relays "my operand is ready / my accumulator is drained" to the leader, which owns the issue loop, and every
-// tcgen05.commit is multicast to the same barrier in both CTAs.
-template <bool X3, bool PAIR>
+// (A CTA-pair version -- every tcgen05.mma issued once for two CTAs' tiles, cta_group::2 -- was bit-identical and not faster,
+// 0.655 vs 0.63-0.67 ms: the instruction count is not the bound, profiles/r02_trunk_fused2.txt.)
+template <bool X3>
 __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t) {
-  static_assert(X3 || !PAIR, "the CTA-pair trunk exists for the three-term split only");
   using S = Trunk2Smem<X3>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -1536,20 +986,14 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
   uint64_t* pl_free = pl_full + 2;                       // [2] conv2 MMAs have read the plane
   uint64_t* tfull = pl_free + 2;                         // [2] accumulator complete
   uint64_t* tempty = tfull + 2;                          // [2] accumulator drained (128 epilogue threads)
-  uint64_t* peer_ready = tempty + 2;                     // [8] PAIR, leader: the peer CTA's c1_full / c1_tfree / pl_full / tempty [2 each]
-  uint64_t* wbar = peer_ready + 8;
+  uint64_t* wbar = tempty + 2;
   uint32_t* tmem_slot = (uint32_t*)(wbar + 1);
-  const uint32_t rank = PAIR ? cluster_ctarank() : 0u;
-  const int64_t unit = PAIR ? (int64_t)(blockIdx.x >> 1) : (int64_t)blockIdx.x;   // scheduling unit: CTA or CTA pair
-  const int64_t n_units = PAIR ? (int64_t)(gridDim.x >> 1) : (int64_t)gridDim.x;
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n = t.n, nn = n * n, rp = n + 1, bp = rp * rp;  // row pitch and board pitch of the shared-border raster
   const int G = (127 - (nn + n - 2)) / bp + 1;                // boards per 128-row tile
   if (t.dyn_rows && *t.dyn_rows < t.B) t.B = *t.dyn_rows;
   const int64_t tiles = (t.B + G - 1) / G;
-  const int64_t tile_units = PAIR ? (tiles + 1) / 2 : tiles;  // a pair owns two consecutive tiles (the second may not exist)
-  auto tile_of = [&](int64_t tp) { return PAIR ? 2 * tp + (int64_t)rank : tp; };
   constexpr int BN = 64;
   constexpr int ACC_COLS = X3 ? 128 : 64;
   constexpr uint32_t TMEM_COLS = 512;
@@ -1557,8 +1001,8 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
 
   for (int i = threadIdx.x; i < 2 * T2_PLANE_BYTES / 16; i += blockDim.x) reinterpret_cast<uint4*>(planes)[i] = make_uint4(0, 0, 0, 0);
   for (int i = threadIdx.x; i < 2 * A_STAGE_BYTES / 16; i += blockDim.x) reinterpret_cast<uint4*>(c1st)[i] = make_uint4(0, 0, 0, 0);
-  for (int i = threadIdx.x; i < (PAIR ? 16 : 32) * 64; i += blockDim.x) {  // conv1 weights as three bf16 terms along K (Connect4Net.py:32)
-    const int row = i >> 6, ch = row + (PAIR ? (int)rank * 16 : 0), col = i & 63, term = col >> 4, k = col & 15;  // PAIR: this CTA's 16 of the 32 rows
+  for (int i = threadIdx.x; i < 32 * 64; i += blockDim.x) {  // conv1 weights as three bf16 terms along K (Connect4Net.py:32)
+    const int ch = i >> 6, col = i & 63, term = col >> 4, k = col & 15;
     float v = 0.0f;
     if (term < 3 && k < 9) {
       const float w = t.w1[ch * 9 + k];
@@ -1566,7 +1010,7 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
       const float mid = __bfloat162float(__float2bfloat16_rn(w - hi));
       v = term == 0 ? hi : term == 1 ? mid : (w - hi) - mid;
     }
-    *reinterpret_cast<__nv_bfloat16*>(w1img + image_offset(row, col)) = __float2bfloat16_rn(v);
+    *reinterpret_cast<__nv_bfloat16*>(w1img + image_offset(ch, col)) = __float2bfloat16_rn(v);
   }
   if (warp == 9 && lane == 0) {
     for (int k = 0; k < 2; ++k) {
@@ -1579,31 +1023,18 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
       mbar_init(&tfull[k], 1);
       mbar_init(&tempty[k], 256);
     }
-    for (int k = 0; k < 8; ++k) mbar_init(&peer_ready[k], 1);
     mbar_init(wbar, 1);
     fence_barrier_init();
   }
-  if (warp == 9) {
-    if (PAIR) tmem_alloc2(tmem_slot, TMEM_COLS);
-    else tmem_alloc(tmem_slot, TMEM_COLS);
-  }
+  if (warp == 9) tmem_alloc(tmem_slot, TMEM_COLS);
   fence_async_smem();
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();  // both CTAs' barriers exist before any remote arrive / multicast commit
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 9) {
-    if (lane == 0 && PAIR) {
-      // this CTA's halves of the two weight operands: rows of [W_hi ; W_lo] (leader: W_hi, peer: W_lo) for the N = 128 product,
-      // rows 32 rank .. 32 rank + 31 of W_hi for the N = 64 product (row groups of 8: contiguous 4 KB of every k-block image)
-      mbar_expect_tx(wbar, TR_W_BYTES + TR_W_BYTES / 2);
-      for (int kb = 0; kb < C2_KB; ++kb) {
-        bulk_g2s(w_s + kb * 8192, (rank == 0 ? t.w_hi : t.w_lo) + kb * 8192, 8192, wbar);
-        bulk_g2s(w_s + TR_W_BYTES + kb * 4096, t.w_hi + kb * 8192 + rank * 4096, 4096, wbar);
-      }
-    } else if (lane == 0) {  // conv2 weight images -> smem, once
+    if (lane == 0) {  // conv2 weight images -> smem, once
       mbar_expect_tx(wbar, (X3 ? 2 : 1) * TR_W_BYTES);
       if (X3) {
         for (int kb = 0; kb < C2_KB; ++kb) {
@@ -1658,18 +1089,17 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
       fence_async_smem();
       mbar_arrive(&c1_full[k]);
     };
-    fetch(tile_of(unit));
-    if (unit < tile_units) c1_operand(0, 0);
-    fetch(tile_of(unit + n_units));
+    fetch(blockIdx.x);
+    if ((int64_t)blockIdx.x < tiles) c1_operand(0, 0);
+    fetch((int64_t)blockIdx.x + gridDim.x);
     uint32_t it = 0;
-    for (int64_t tp = unit; tp < tile_units; tp += n_units, ++it) {
-      const int64_t tile = tile_of(tp);
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
       const int k = (int)(it & 1u);
       const uint32_t ph = (it >> 1) & 1u;
-      const bool has_next = tp + n_units < tile_units;
+      const bool has_next = tile + gridDim.x < tiles;
       if (has_next) {  // the next tile's conv1 operand depends on nothing the tensor core produces: build it first, so that
         c1_operand(k ^ 1, it + 1);  // conv1(it+1) is queued before conv2(it) and only the plane write-back below sits
-        fetch(tile_of(tp + 2 * n_units));  // between a conv1 result and the conv2 MMAs that need it
+        fetch(tile + 2 * (int64_t)gridDim.x);  // between a conv1 result and the conv2 MMAs that need it
       }
       mbar_wait(&c1_done[k], ph);
       tc_fence_after();
@@ -1700,98 +1130,57 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
     }
   } else if (warp == 8) {
     // ======================= MMA issuer =======================
-    if (lane == 0 && rank != 0) {
-      // peer CTA of a pair: forward this CTA's "ready" events to the leader, in the order the leader waits for them
-      mbar_wait(wbar, 0);  // (keeps the weight copies of this CTA inside the kernel's lifetime before the first relay)
-      const uint32_t leader = map_to_cta(&peer_ready[0], 0);
-      auto relay = [&](uint64_t* local, uint32_t parity, int slot) {
-        mbar_wait(local, parity);
-        mbar_arrive_cluster(leader + (uint32_t)slot * 8u);
-      };
-      if (unit < tile_units) {
-        relay(&c1_full[0], 0u, 0);
-        relay(&c1_tfree[0], 1u, 2);
-      }
-      uint32_t it = 0;
-      for (int64_t tp = unit; tp < tile_units; tp += n_units, ++it) {
-        const int k = (int)(it & 1u);
-        const uint32_t ph = (it >> 1) & 1u, phn = ((it + 1) >> 1) & 1u;
-        if (tp + n_units < tile_units) {
-          relay(&c1_full[k ^ 1], phn, 0 + (k ^ 1));
-          relay(&c1_tfree[k ^ 1], phn ^ 1u, 2 + (k ^ 1));
-        }
-        relay(&pl_full[k], ph, 4 + k);
-        relay(&tempty[k], ph ^ 1u, 6 + k);
-      }
-    } else if (lane == 0) {
-      constexpr uint32_t idesc = make_idesc(PAIR ? 2 * BM : BM, BN);
-      constexpr uint32_t idesc_c1 = make_idesc(PAIR ? 2 * BM : BM, 32);
-      constexpr uint32_t idesc_cat = make_idesc(PAIR ? 2 * BM : BM, 2 * BN);
-      auto mma = [&](uint32_t d, uint64_t a, uint64_t b, uint32_t id, uint32_t acc) {
-        if (PAIR) umma2_bf16(d, a, b, id, acc);
-        else umma_bf16(d, a, b, id, acc);
-      };
-      auto commit = [&](uint64_t* bar) {
-        if (PAIR) umma2_commit(bar);
-        else umma_commit(bar);
-      };
+    if (lane == 0) {
+      constexpr uint32_t idesc = make_idesc(BM, BN);
+      constexpr uint32_t idesc_c1 = make_idesc(BM, 32);
+      constexpr uint32_t idesc_cat = make_idesc(BM, 2 * BN);
       mbar_wait(wbar, 0);
       const uint32_t w_addr = smem_u32(w_s);
       const uint64_t b_c1 = make_smem_desc(smem_u32(w1img));
       auto conv1 = [&](int k, uint32_t it) {  // [A | A | A] x [w_hi | w_mid | w_lo]^T -> conv1 region k
         mbar_wait(&c1_full[k], (it >> 1) & 1u);
-        if (PAIR) mbar_wait_cluster(&peer_ready[0 + k], (it >> 1) & 1u);
         mbar_wait(&c1_tfree[k], ((it >> 1) & 1u) ^ 1u);  // the builders have read the region's previous content
-        if (PAIR) mbar_wait_cluster(&peer_ready[2 + k], (it >> 1) & 1u);
         tc_fence_after();
         const uint64_t a_c1 = make_smem_desc(smem_u32(c1st + k * A_STAGE_BYTES));
 #pragma unroll
-        for (int q = 0; q < 3; ++q) mma(tmem_base + C1_COL + (uint32_t)(k * 32), a_c1 + 2 * q, b_c1 + 2 * q, idesc_c1, q != 0);
-        commit(&c1_free[k]);
-        commit(&c1_done[k]);
+        for (int q = 0; q < 3; ++q) umma_bf16(tmem_base + C1_COL + (uint32_t)(k * 32), a_c1 + 2 * q, b_c1 + 2 * q, idesc_c1, q != 0);
+        umma_commit(&c1_free[k]);
+        umma_commit(&c1_done[k]);
       };
-      if (unit < tile_units) conv1(0, 0);
+      if ((int64_t)blockIdx.x < tiles) conv1(0, 0);
       // descriptor increments of the nine taps in 16-byte units (the single issuing thread should spend its cycles on
       // tcgen05.mma, not on address arithmetic: everything but two additions per step is hoisted or a constant)
       uint32_t tap16[9];
 #pragma unroll
       for (int q = 0; q < 9; ++q) tap16[q] = (uint32_t)((q / 3) * rp + (q % 3)) * 8u;
       const uint64_t b_base = make_smem_desc(w_addr);
-      const uint64_t b_half = make_smem_desc(w_addr + TR_W_BYTES);  // PAIR: this CTA's 32 rows of W_hi
       const uint64_t a_base[2] = {make_smem_desc(smem_u32(planes)), make_smem_desc(smem_u32(planes + T2_PLANE_BYTES))};
       uint32_t it = 0;
-      for (int64_t tp = unit; tp < tile_units; tp += n_units, ++it) {
+      for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
         const int k = (int)(it & 1u);
         const uint32_t ph = (it >> 1) & 1u;
-        if (tp + n_units < tile_units) conv1(k ^ 1, it + 1);  // before this tile's conv2: its write-back overlaps the 36 MMAs
+        if (tile + gridDim.x < tiles) conv1(k ^ 1, it + 1);  // before this tile's conv2: its write-back overlaps the 36 MMAs
         mbar_wait(&pl_full[k], ph);
-        if (PAIR) mbar_wait_cluster(&peer_ready[4 + k], ph);
         mbar_wait(&tempty[k], ph ^ 1u);
-        if (PAIR) mbar_wait_cluster(&peer_ready[6 + k], ph);
         tc_fence_after();
         const uint32_t d_tmem = tmem_base + (uint32_t)(k * ACC_COLS);
 #pragma unroll
         for (int s = 0; s < 18; ++s) {
           // base-offset field of the shifted descriptor stays 0 (see the header comment)
           const uint64_t a_hi = a_base[k] + (uint64_t)(tap16[s >> 1] + (uint32_t)(s & 1) * 2u);
-          if (PAIR) {  // each CTA supplies half of the weight rows: 64 of [W_hi ; W_lo], 32 of W_hi
-            mma(d_tmem, a_hi, b_base + (uint64_t)((s >> 2) * (64 * 128 / 16) + 2 * (s & 3)), idesc_cat, s != 0);
-            mma(d_tmem + BN, a_hi + 4, b_half + (uint64_t)((s >> 2) * (32 * 128 / 16) + 2 * (s & 3)), idesc, 1);
-            continue;
-          }
           const uint64_t b_w = b_base + (uint64_t)((s >> 2) * (X3 ? 2 : 1) * (64 * 128 / 16) + 2 * (s & 3));
           if (X3) {
             // Both correction products go to columns 64-127: the tensor core's fp32 accumulation truncates once per MMA
             // by up to an ulp OF THE ACCUMULATOR, so small terms added to the large hi x W_hi sum would double its
             // truncation bias (36 instead of 18 accumulations); among themselves they cost nothing measurable.
-            mma(d_tmem, a_hi, b_w, idesc_cat, s != 0);           // hi x [W_hi ; W_lo]: columns 0-63 and 64-127
-            mma(d_tmem + BN, a_hi + 4, b_w, idesc, 1);           // lo (64 bytes further in the cell) x W_hi: columns 64-127
+            umma_bf16(d_tmem, a_hi, b_w, idesc_cat, s != 0);     // hi x [W_hi ; W_lo]: columns 0-63 and 64-127
+            umma_bf16(d_tmem + BN, a_hi + 4, b_w, idesc, 1);     // lo (64 bytes further in the cell) x W_hi: columns 64-127
           } else {
-            mma(d_tmem, a_hi, b_w, idesc, s != 0);
+            umma_bf16(d_tmem, a_hi, b_w, idesc, s != 0);
           }
         }
-        commit(&pl_free[k]);
-        commit(&tfull[k]);
+        umma_commit(&pl_free[k]);
+        umma_commit(&tfull[k]);
       }
     }
   } else if (warp >= 12) {
@@ -1820,8 +1209,7 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
     }
     const bool f8 = X3 && t.out_f8;
     uint32_t it = 0;
-    for (int64_t tp = unit; tp < tile_units; tp += n_units, ++it) {
-      const int64_t tile = tile_of(tp);
+    for (int64_t tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
       const int k = (int)(it & 1u);
       const int rb = (int)((tile * G + r / bp) & 127);  // image row (board & 127) of this thread's tile row
       mbar_wait(&tfull[k], (it >> 1) & 1u);
@@ -1889,42 +1277,27 @@ __global__ void __launch_bounds__(T2_THREADS, 1) c4_trunk2_tc_kernel(TrunkArgs t
 
   tc_fence_before();
   __syncthreads();
-  if (PAIR) cluster_sync_all();  // the leader's MMAs read the peer's shared memory: leave together
   if (warp == 9) {
     tc_fence_after();
-    if (PAIR) tmem_dealloc2(tmem_base, TMEM_COLS);
-    else tmem_dealloc(tmem_base, TMEM_COLS);
+    tmem_dealloc(tmem_base, TMEM_COLS);
   }
 }
 
-template <bool X3, bool PAIR>
+template <bool X3>
 int launch_trunk2(const TrunkArgs& t, cudaStream_t st) {
   static bool configured = false;
   int dev = 0, sms = 0;
   AZG_CUDA_CHECK(cudaGetDevice(&dev));
   AZG_CUDA_CHECK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
   if (!configured) {
-    AZG_CUDA_CHECK(cudaFuncSetAttribute(c4_trunk2_tc_kernel<X3, PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, Trunk2Smem<X3>::TOTAL));
+    AZG_CUDA_CHECK(cudaFuncSetAttribute(c4_trunk2_tc_kernel<X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, Trunk2Smem<X3>::TOTAL));
     configured = true;
   }
   const int n = t.n, bp = (n + 1) * (n + 1);
   const int G = (127 - (n * n + n - 2)) / bp + 1;
   const int64_t tiles = (t.B + G - 1) / G;
-  const int64_t units = PAIR ? (tiles + 1) / 2 : tiles, max_units = PAIR ? sms / 2 : sms;
-  const int grid = (int)(units < max_units ? units : max_units) * (PAIR ? 2 : 1);
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(T2_THREADS);
-  cfg.dynamicSmemBytes = Trunk2Smem<X3>::TOTAL;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = PAIR ? 2 : 1;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  AZG_CUDA_CHECK(cudaLaunchKernelEx(&cfg, c4_trunk2_tc_kernel<X3, PAIR>, t));
+  const int grid = (int)(tiles < sms ? tiles : sms);
+  c4_trunk2_tc_kernel<X3><<<grid, T2_THREADS, Trunk2Smem<X3>::TOTAL, st>>>(t);
   AZG_LAUNCH_CHECK();
   return AZG_OK;
 }
@@ -1939,10 +1312,10 @@ int make_image(const float* src, int64_t rows, int64_t rows_padded, int K, int R
 // ---------------------------------------------------------------------------------------------
 // Packed weight blob of the tensor-core Connect4 path (azg_c4_pack), sections 1024-B aligned:
 //   W0 (output_transform.0, input order permuted to the feature image) hi [lo]
-//   W2 (output_transform.2) hi [lo] | conv2 [64 x 320] hi [lo] | head weights permuted, fp32
+//   W2 (output_transform.2) hi [lo] | conv2 [64 x 320] hi [lo] | head weights (fp32, and as a weight image) | folded heads
 namespace {
 struct PackLayout {
-  size_t w0_hi, w0_lo, w2_hi, w2_lo, c2_hi, c2_lo, heads, heads_cat, hd_hi, hd_lo, bias32, fold_w, fold_b, scales, total;
+  size_t w0_hi, w0_lo, w2_hi, w2_lo, c2_hi, c2_lo, heads_cat, hd_hi, hd_lo, bias32, fold_w, fold_b, scales, total;
   bool x3, gnn, f8;  // x3: hi + lo images (bf16x3 and the fp16+FP8 split); f8: the latter
 };
 // AZG_PREC_F16F8_KS runs on the operand images of AZG_PREC_F16F8 (same packed blob, same tile widths); it differs in how
@@ -1983,7 +1356,6 @@ PackLayout pack_layout(int n, int prec, bool gnn) {
   }
   L.c2_hi = take(cimg);
   L.c2_lo = L.x3 ? take(cimg) : 0;
-  L.heads = take((size_t)(n + 2) * F * 4);      // permuted to the feature image order (std heads)
   L.heads_cat = take((size_t)32 * F * 4);       // reference order, zero-padded to 32 rows (GEMM-2 epilogue)
   L.hd_hi = take((size_t)32 * F * 2);           // std heads as a [32 x F] weight image (feature-image order)
   L.hd_lo = L.x3 ? take((size_t)32 * F * 2) : 0;
@@ -1996,7 +1368,7 @@ PackLayout pack_layout(int n, int prec, bool gnn) {
 }
 
 struct ScratchLayout {
-  size_t a2_hi, a2_lo, f_hi, f_lo, h_hi, h_lo, part, lg32, acc, total;
+  size_t f_hi, f_lo, h_hi, h_lo, part, lg32, acc, total;
 };
 
 ScratchLayout scratch_layout(int n, int64_t B, int prec, bool gnn) {
@@ -2005,12 +1377,10 @@ ScratchLayout scratch_layout(int n, int64_t B, int prec, bool gnn) {
   prec = prec_base(prec);
   const bool x3 = prec == AZG_PREC_BF16X3 || prec == AZG_PREC_F16F8;
   const size_t nn = (size_t)n * n, F = 64 * nn;
-  const size_t M2p = (size_t)azg_ceil_div(B * (int64_t)nn, tc::BM) * tc::BM, Mp = (size_t)azg_ceil_div(B, 2 * tc::BM) * 2 * tc::BM;  // even number of m-tiles (CTA pairs)
-  const size_t a2 = M2p * tc::C2_K * 2, fimg = Mp * F * 2;
+  const size_t Mp = (size_t)azg_ceil_div(B, 2 * tc::BM) * 2 * tc::BM;  // even number of m-tiles (CTA pairs)
+  const size_t fimg = Mp * F * 2;
   size_t off = 0;
   auto take = [&](size_t bytes) { size_t o = off; off = up1k(off + bytes); return o; };
-  S.a2_hi = take(a2);
-  S.a2_lo = x3 ? take(a2) : 0;
   S.f_hi = take(fimg);
   S.f_lo = x3 ? take(fimg) : 0;
   S.lg32 = take(Mp * 32 * sizeof(float));
@@ -2028,37 +1398,10 @@ ScratchLayout scratch_layout(int n, int64_t B, int prec, bool gnn) {
 }
 }  // namespace
 
-static int azg_trunk_mode() {  // 0 = fused (either generation), 1 = split (im2col through HBM; A/B measurements)
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("AZG_TRUNK");
-    mode = (e && strcmp(e, "split") == 0) ? 1 : 0;
-  }
-  return mode;
-}
-
-static int azg_trunk_gen() {  // AZG_TRUNK=fused1: the first-generation fused trunk (patch copies); fused2pair: generation 2 on
-  static int gen = -1;        // CTA pairs (cta_group::2) -- both kept for A/B measurements (profiles/r02_trunk_fused2.txt)
-  if (gen < 0) {
-    const char* e = getenv("AZG_TRUNK");
-    gen = (e && strcmp(e, "fused1") == 0) ? 1 : (e && strcmp(e, "fused2pair") == 0) ? 3 : 2;
-  }
-  return gen;
-}
-
-static int azg_std_heads_mode() {  // AZG_STD_HEADS=split: predict's heads in their own skinny GEMM launch (A/B measurements)
-  static int mode = -1;
-  if (mode < 0) {
-    const char* e = getenv("AZG_STD_HEADS");
-    mode = (e && strcmp(e, "split") == 0) ? 1 : 0;
-  }
-  return mode;
-}
-
 size_t azg_tc_scratch_bytes(int n, int64_t B, int prec) { return scratch_layout(n, B, prec, true).total; }
 
-// Whole Connect4 leaf evaluation on the tensor-core path: im2col(encode+conv1) -> conv2 GEMM ->
-// [std heads] -> [output_transform GEMMs -> enh fp32 for the GNN heads].
+// Whole Connect4 leaf evaluation on the tensor-core path: fused trunk (encode + conv1 + conv2) -> feature image ->
+// [std heads] -> [output_transform GEMMs -> fused GNN heads].
 int azg_tc_c4_forward(const void* packed, const azg_c4_params* p, int n, int prec, const uint64_t* states, int64_t B,
                       int eval_mask, float* pi_std, float* v_std, float* pi_gnn, float* v_gnn, void* scratch,
                       size_t scratch_bytes, const int32_t* dyn_rows, cudaStream_t st) {
@@ -2068,12 +1411,10 @@ int azg_tc_c4_forward(const void* packed, const azg_c4_params* p, int n, int pre
   const ScratchLayout S = scratch_layout(n, B, prec, true);
   prec = prec_base(prec);
   const bool f8 = prec == AZG_PREC_F16F8, x3 = prec == AZG_PREC_BF16X3 || f8, gnn = (eval_mask & AZG_EVAL_GNN) != 0;
-  AZG_REQUIRE(!f8 || azg_trunk_mode() == 0, "tcgen05 path: the fp16+FP8 split needs the fused trunk (unset AZG_TRUNK)");
   const PackLayout L = pack_layout(n, prec, true);
   AZG_REQUIRE(scratch && scratch_bytes >= S.total, "tcgen05 path: scratch %zu < %zu", scratch_bytes, S.total);
   uint8_t* sc = (uint8_t*)(((uintptr_t)scratch + 1023) & ~(uintptr_t)1023);
   const uint8_t* w = (const uint8_t*)packed;
-  uint8_t *a2_hi = sc + S.a2_hi, *a2_lo = x3 ? sc + S.a2_lo : nullptr;
   uint8_t *f_hi = sc + S.f_hi, *f_lo = x3 ? sc + S.f_lo : nullptr;
   uint8_t *h_hi = sc + S.h_hi, *h_lo = x3 ? sc + S.h_lo : nullptr;
   int rc;
@@ -2109,41 +1450,22 @@ int azg_tc_c4_forward(const void* packed, const azg_c4_params* p, int n, int pre
     return AZG_OK;
   };
   azg_phase_begin(AZG_PHASE_TRUNK, st);
-  tc::GemmArgs g{};
-  if (azg_trunk_mode() == 0) {  // fused: encode + conv1 + im2col in smem -> tcgen05 conv2
-    tc::TrunkArgs t{};
-    t.states = states; t.w1 = p->conv1_w; t.b1 = p->conv1_b; t.b2 = p->conv2_b;
-    t.w_hi = w + L.c2_hi; t.w_lo = x3 ? w + L.c2_lo : nullptr; t.f_hi = f_hi; t.f_lo = f_lo; t.B = B; t.n = n;
-    t.dyn_rows = dyn_rows;
-    t.out_f8 = f8 ? 1 : 0;
-    if (azg_trunk_gen() == 1) rc = x3 ? tc::launch_trunk<true>(t, st) : tc::launch_trunk<false>(t, st);
-    else if (!x3) rc = tc::launch_trunk2<false, false>(t, st);
-    else rc = azg_trunk_gen() == 3 ? tc::launch_trunk2<true, true>(t, st) : tc::launch_trunk2<true, false>(t, st);
-    if (rc) return rc;
-  } else {  // split: im2col image through HBM, conv2 on the generic GEMM kernel (kept for A/B measurements)
-    const int grid = (int)(B < 148 * 8 ? B : 148 * 8);
-    tc::c4_im2col_kernel<<<grid, 256, 0, st>>>(states, n, B, p->conv1_w, p->conv1_b, a2_hi, a2_lo);
-    AZG_LAUNCH_CHECK();
-    g.M = B * (int64_t)nn;
-    g.m_tiles = (int)azg_ceil_div(g.M, tc::BM);
-    g.n_tiles = 1;
-    g.KB = tc::C2_KB;
-    g.x3 = x3;
-    g.a_hi = a2_hi; g.a_lo = a2_lo; g.w_hi = w + L.c2_hi; g.w_lo = x3 ? w + L.c2_lo : nullptr;
-    g.bias = p->conv2_b; g.relu = 1; g.out_mode = x3 ? tc::OUT_FEAT_HILO : tc::OUT_FEAT; g.feat_nn = nn;
-    g.out_hi = f_hi; g.out_lo = f_lo; g.dyn_rows = dyn_rows;
-    if ((rc = tc::run_gemm(64, g, st))) return rc;
-  }
+  tc::TrunkArgs t{};
+  t.states = states; t.w1 = p->conv1_w; t.b1 = p->conv1_b; t.b2 = p->conv2_b;
+  t.w_hi = w + L.c2_hi; t.w_lo = x3 ? w + L.c2_lo : nullptr; t.f_hi = f_hi; t.f_lo = f_lo; t.B = B; t.n = n;
+  t.dyn_rows = dyn_rows;
+  t.out_f8 = f8 ? 1 : 0;
+  rc = x3 ? tc::launch_trunk2<true>(t, st) : tc::launch_trunk2<false>(t, st);
+  if (rc) return rc;
   azg_phase_end(AZG_PHASE_TRUNK, st);
-  // predict's heads ride on GEMM-1 as a side tile when the CTA-pair kernel runs it (AZG_STD_HEADS=split: own launch)
+  // predict's heads ride on GEMM-1 as a side tile
   const int32_t* scales = (const int32_t*)(w + L.scales);
-  const bool std_side = (eval_mask & AZG_EVAL_STD) && azg_trunk_mode() == 0 &&
-                        (f8 || (tc::gemm_pair_mode() && BN >= 128 && azg_std_heads_mode() == 0));
+  const bool std_side = (eval_mask & AZG_EVAL_STD) != 0;
   if (std_side && !gnn) {  // std only: the same side-tile code with no main n-tiles (bit-identical to the combined call)
     AZG_REQUIRE(pi_std && v_std && A <= 9, "tcgen05 path: bad std outputs");
     azg_phase_begin(AZG_PHASE_HEADS, st);
     tc::GemmArgs h{};
-    h.M = B; h.m_tiles = (int)azg_ceil_div(B, tc::BM); h.n_tiles = 0; h.KB = F / tc::BK; h.x3 = x3; h.pair_ok = 1;
+    h.M = B; h.m_tiles = (int)azg_ceil_div(B, tc::BM); h.n_tiles = 0; h.KB = F / tc::BK; h.x3 = x3;
     h.a_hi = f_hi; h.a_lo = f_lo; h.dyn_rows = dyn_rows;
     h.side_hi = w + L.hd_hi; h.side_lo = x3 ? w + L.hd_lo : nullptr;
     h.side_bias = (const float*)(w + L.bias32); h.side_out = (float*)(sc + S.lg32);
@@ -2154,35 +1476,14 @@ int azg_tc_c4_forward(const void* packed, const azg_c4_params* p, int n, int pre
     azg_phase_end(AZG_PHASE_HEADS, st);
     return AZG_OK;
   }
-  if ((eval_mask & AZG_EVAL_STD) && !std_side) {
-    AZG_REQUIRE(pi_std && v_std && A <= 9, "tcgen05 path: bad std outputs");
-    azg_phase_begin(AZG_PHASE_HEADS, st);
-    if (azg_trunk_mode() == 0) {  // predict's heads (Connect4Net.py:55-60) as a skinny tcgen05 GEMM: [B,F] x [F,32]
-      tc::GemmArgs h{};
-      h.M = B; h.m_tiles = (int)azg_ceil_div(B, tc::BM); h.n_tiles = 1; h.KB = F / tc::BK; h.x3 = x3;
-      h.a_hi = f_hi; h.a_lo = f_lo; h.w_hi = w + L.hd_hi; h.w_lo = x3 ? w + L.hd_lo : nullptr;
-      h.bias = (const float*)(w + L.bias32); h.relu = 0; h.out_mode = tc::OUT_F32; h.out_f32 = (float*)(sc + S.lg32);
-      h.dyn_rows = dyn_rows;
-      if ((rc = tc::run_gemm(32, h, st))) return rc;
-      tc::heads32_finalize_kernel<<<(unsigned)((B + 127) / 128), 128, 0, st>>>((const float*)(sc + S.lg32), A, B, dyn_rows, pi_std, v_std);
-      AZG_LAUNCH_CHECK();
-    } else {
-      const int grid = (int)(azg_ceil_div(B, 8) < 148 * 8 ? azg_ceil_div(B, 8) : 148 * 8);
-      tc::heads_image_kernel<9><<<grid, 256, 0, st>>>(f_hi, f_lo, nn, (const float*)(w + L.heads), p->fc_policy_b,
-                                                      p->fc_value_b, A, B, pi_std, v_std);
-      AZG_LAUNCH_CHECK();
-    }
-    azg_phase_end(AZG_PHASE_HEADS, st);
-  }
   if (!gnn) return AZG_OK;
   azg_phase_begin(AZG_PHASE_GEMM, st);
-  g = tc::GemmArgs{};
+  tc::GemmArgs g{};
   g.M = B;
   g.m_tiles = (int)azg_ceil_div(B, tc::BM);
   g.n_tiles = F / BN;
   g.KB = F / tc::BK;
   g.x3 = x3;
-  g.pair_ok = 1;
   g.dyn_rows = dyn_rows;
   g.a_hi = f_hi; g.a_lo = f_lo; g.w_hi = w + L.w0_hi; g.w_lo = x3 ? w + L.w0_lo : nullptr; g.bias = p->ot0_b; g.relu = 1;
   g.f8 = f8 ? tc::f8_terms() : 0; g.w_exp = scales + 0; g.side_exp = scales + 2;
@@ -2266,9 +1567,6 @@ int azg_c4_pack(const azg_c4_params* p, int n, int prec, void* packed, size_t pa
     if (rc) return rc;
   }
   tc::conv2_weight_image_kernel<<<(64 * (tc::C2_K / 8) + 127) / 128, 128, 0, st>>>(p->conv2_w, w + L.c2_hi, x3 ? w + L.c2_lo : nullptr);
-  AZG_LAUNCH_CHECK();
-  const int64_t hn = (int64_t)(A + 1) * F;
-  tc::permute_heads_kernel<<<(unsigned)((hn + 255) / 256), 256, 0, st>>>(p->fc_policy_w, p->fc_value_w, A, F, nn, (float*)(w + L.heads));
   AZG_LAUNCH_CHECK();
   tc::concat_heads_kernel<<<(unsigned)(((int64_t)32 * F + 255) / 256), 256, 0, st>>>(
       p->fc_policy_w, p->fc_value_w, p->fc_policy_b, p->fc_value_b, A, F, (float*)(w + L.heads_cat), (float*)(w + L.bias32));
@@ -2402,7 +1700,6 @@ int ttt_gemm(const uint8_t* a_hi, const uint8_t* a_lo, int64_t M, const TttLayer
              bool x3, float* C, cudaStream_t st) {
   tc::GemmArgs g{};
   g.M = M; g.m_tiles = (int)azg_ceil_div(M, tc::BM); g.n_tiles = l.N / l.BN; g.KB = l.Kp / tc::BK; g.x3 = x3;
-  g.pair_ok = l.BN == 256 ? 1 : 0;
   g.a_hi = a_hi; g.a_lo = x3 ? a_lo : nullptr; g.w_hi = w + l.hi; g.w_lo = x3 ? w + l.lo : nullptr; g.bias = bias; g.relu = relu;
   g.out_mode = tc::OUT_F32; g.out_f32 = C;
   return tc::run_gemm(l.BN, g, st);
@@ -2547,7 +1844,7 @@ int azg_tc_linear(const float* A, const float* W, const float* bias, float* C, i
   if ((rc = tc::to_image(W, F, F, F, BN, w_hi, w_lo, st, f8 ? 2 : 0, scales))) return rc;
   tc::GemmArgs g{};
   g.f8 = f8 ? tc::f8_terms() : 0; g.w_exp = scales;
-  g.M = M; g.m_tiles = (int)m_tiles; g.n_tiles = F / BN; g.KB = F / tc::BK; g.x3 = x3; g.pair_ok = 1;
+  g.M = M; g.m_tiles = (int)m_tiles; g.n_tiles = F / BN; g.KB = F / tc::BK; g.x3 = x3;
   g.a_hi = a_hi; g.a_lo = a_lo; g.w_hi = w_hi; g.w_lo = w_lo; g.bias = bias; g.relu = relu;
   g.out_mode = tc::OUT_F32; g.out_f32 = C;
   if (ks > 1 && !ksplit_by_launches()) {

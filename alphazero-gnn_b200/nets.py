@@ -310,7 +310,7 @@ class B200Connect4NNetWrapper(_TwoPlayer):
         return p
 
     def _ensure_packed(self, prec, params):
-        """tcgen05 operand images of the weights (conv2, output_transform, permuted heads), one blob
+        """tcgen05 operand images of the weights (conv2, output_transform, heads), one blob
         per precision, rebuilt lazily after weights_changed()."""
         prec = _lib.PACKED_AS.get(prec, prec)
         if not self._packed_ok:

@@ -126,7 +126,7 @@ int azg_c4_forward(const azg_c4_params* p, int n, const uint64_t* states, int64_
 int azg_c4_forward_dyn(const azg_c4_params* p, int n, const uint64_t* states, int64_t B, const int32_t* dyn_rows,
                        int eval_mask, int prec, float* pi_std, float* v_std, float* pi_gnn, float* v_gnn,
                        void* workspace, size_t workspace_bytes, azg_stream stream);
-/* Build the tcgen05 operand images of the weights (conv2, output_transform, permuted heads) for
+/* Build the tcgen05 operand images of the weights (conv2, output_transform, heads) for
  * AZG_PREC_BF16X3 / AZG_PREC_BF16 / AZG_PREC_F16F8 (AZG_PREC_F16F8_KS / AZG_PREC_BF16X3_KS read the AZG_PREC_F16F8 / AZG_PREC_BF16X3 images and may be passed
  * instead: same bytes); the result goes into azg_c4_params.ot_packed.  Call again after
  * every optimizer step / load_checkpoint.  packed: device memory, 16-byte aligned. */

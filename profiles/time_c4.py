@@ -1,5 +1,6 @@
 """Step time of the Connect4 leaf evaluation (65,536 positions, std + GNN predictions) per precision, with the library's
-phase timers (trunk / GEMMs / heads).  usage: python profiles/time_c4.py [precisions...]; env switches apply (A/B runs)."""
+phase timers (trunk / GEMMs / heads).  usage: python profiles/time_c4.py [precisions...]; AZG_LIBRARY selects the build
+(A/B runs), AZG_KSPLIT and AZG_F8_TERMS apply."""
 import ctypes as C
 import os
 import sys
@@ -40,5 +41,5 @@ for prec in precs:
         lib.azg_timing_read(i, C.byref(d), C.byref(n))
         ph.append(d.value / max(n.value, 1))
     lib.azg_timing_enable(0)
-    print(f"{prec:14s} opt={os.environ.get('AZG_GEMM_OPT', '-'):6s} {ms:7.3f} ms/step = {65536 / ms / 1e3:6.2f} M leaf evals/s   phases (trunk, gemm, heads) ms: "
+    print(f"{prec:14s} {ms:7.3f} ms/step = {65536 / ms / 1e3:6.2f} M leaf evals/s   phases (trunk, gemm, heads) ms: "
           + " ".join(f"{x:.3f}" for x in ph), flush=True)

@@ -1,4 +1,4 @@
-"""Numerics of the fused trunk's tensor-core conv1 (csrc/azg_gemm_tc.cu, c4_trunk_tc_kernel), restated in torch on the CPU:
+"""Numerics of the fused trunk's tensor-core conv1 (csrc/azg_gemm_tc.cu, c4_trunk2_tc_kernel), restated in torch on the CPU:
 the 3x3 neighbourhood of a cell is an exact bf16 operand in {-1, 0, +1}, the fp32 weight is the sum of three bf16 terms,
 products are exact and accumulation is fp32 -- so conv1 on the tensor core reproduces Connect4Net.py:45 to fp32 rounding."""
 import numpy as np
