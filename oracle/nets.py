@@ -150,7 +150,7 @@ def fl_forward(p, node_boards, num_layers):
     x = node_boards.reshape(k, -1)
     x = F.relu(F.linear(x, p["feature_extractor.0.weight"], p["feature_extractor.0.bias"]))
     x = F.relu(F.linear(x, p["feature_extractor.2.weight"], p["feature_extractor.2.bias"]))
-    adj = fl_adjacency(k)
+    adj = fl_adjacency(k).to(x.dtype)
     for l in range(num_layers):
         sup = F.linear(x, p[f"gnn_layers.{l}.W.weight"], p[f"gnn_layers.{l}.W.bias"])
         x = F.relu(torch.mm(adj, sup))
