@@ -782,49 +782,75 @@ __device__ __forceinline__ float grid_deg_inv_sqrt(int x, int y, int gh, int gw)
   return 1.0f / sqrtf((float)deg);
 }
 
+constexpr int GRID_AGG_CHUNK = 256;              // nodes per neighbour table (10 KB of shared memory)
+constexpr int64_t GRID_AGG_MAX_NODES = 1 << 30;  // node indices, node chunks and gh * gw stay inside int
+
+// The loads of a thread's <= 5 neighbours are all issued before the first FMA, and the backward is held to 4 CTAs per SM
+// (<= 64 registers).  Measured on an NVIDIA B200 at its 1,000 W power limit, aggregation alone, against the kernel that
+// had no node chunks (both builds alternating within one run; GB/s of the fp32 rows of bench_sweep.py or of 20 timed
+// launches on working sets above L2):
+//  - with the chunk loop but loads interleaved with the FMAs (the compiler's schedule of the plain loop), the forward
+//    dropped from 4,405-4,413 to 4,068-4,091 GB/s at 7x7, H = 128, B = 16,384 and from 4,620 to 4,184-4,194 at 16x16;
+//  - loads first without the CTA bound, the backward took 80 registers (3 CTAs per SM) and fell from 2,972-2,993 to
+//    2,405-2,466 GB/s at 3x3, H = 64, B = 131,072 (one pass of the node loop per graph);
+//  - as written: forward 4,636-4,645 (was 4,448-4,454) at 7x7 and 4,733-4,737 (4,589-4,594) at 16x16, H = 128;
+//    backward 4,325-4,359 (3,852-3,877) at 16x16, H = 256, and 2,936-2,969 (2,947-2,952) at 3x3, H = 64.
 template <bool BWD>
-__global__ void __launch_bounds__(256) grid_aggregate_kernel(const float* __restrict__ in, const float* __restrict__ act,
+__global__ void __launch_bounds__(256, BWD ? 4 : 0) grid_aggregate_kernel(const float* __restrict__ in, const float* __restrict__ act,
                                                              int64_t B, int gh, int gw, int H, float* __restrict__ out) {
   // FWD: out = relu(adj * in).            BWD: out = adj^T * (in * (act > 0)) = adj * (...), adj symmetric
   // Thread layout: x = 4-channel group, y = node slot; a CTA walks whole graphs.  The <= 5 (neighbour,
-  // coefficient) pairs of every node are tabulated once per CTA in shared memory, so the streaming loop is
+  // coefficient) pairs of every node are tabulated per CTA in shared memory, so the streaming loop is
   // index-math free: per output float4 at most five 128-bit loads (neighbours of a graph hit L1) and one store.
-  __shared__ int16_t nb_idx[256 * 5];
-  __shared__ float nb_coef[256 * 5];
+  // The table holds GRID_AGG_CHUNK nodes: larger graphs are walked one node chunk at a time, each chunk over all of
+  // the CTA's graphs (graphs of up to GRID_AGG_CHUNK nodes: one chunk, the table is filled once).
+  __shared__ int32_t nb_idx[GRID_AGG_CHUNK * 5];
+  __shared__ float nb_coef[GRID_AGG_CHUNK * 5];
   const int H4 = H >> 2, n = gh * gw;
   const int tid = threadIdx.y * blockDim.x + threadIdx.x;
-  for (int i = tid; i < n * 5; i += blockDim.x * blockDim.y) {
-    const int node = i / 5, k = i % 5, x = node / gw, y = node % gw;
-    const int dx = (k == 1) ? -1 : (k == 2) ? 1 : 0, dy = (k == 3) ? -1 : (k == 4) ? 1 : 0;
-    const int nx = x + dx, ny = y + dy;
-    const bool ok = nx >= 0 && nx < gh && ny >= 0 && ny < gw;
-    nb_idx[i] = ok ? (int16_t)(nx * gw + ny) : (int16_t)-1;
-    nb_coef[i] = ok ? grid_deg_inv_sqrt(x, y, gh, gw) * grid_deg_inv_sqrt(nx, ny, gh, gw) : 0.0f;
-  }
-  __syncthreads();
   const float4* in4 = reinterpret_cast<const float4*>(in);
   const float4* act4 = reinterpret_cast<const float4*>(act);
   float4* out4 = reinterpret_cast<float4*>(out);
-  for (int64_t b = blockIdx.x; b < B; b += gridDim.x) {
-    const int64_t g0 = b * n;
-    for (int node = threadIdx.y; node < n; node += blockDim.y) {
-      for (int c4 = threadIdx.x; c4 < H4; c4 += blockDim.x) {
-        float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int base = 0; base < n; base += GRID_AGG_CHUNK) {
+    const int cn = min(n - base, GRID_AGG_CHUNK);
+    if (base > 0) __syncthreads();  // every thread is done reading the previous chunk's table
+    for (int i = tid; i < cn * 5; i += blockDim.x * blockDim.y) {
+      const int node = base + i / 5, k = i % 5, x = node / gw, y = node % gw;
+      const int dx = (k == 1) ? -1 : (k == 2) ? 1 : 0, dy = (k == 3) ? -1 : (k == 4) ? 1 : 0;
+      const int nx = x + dx, ny = y + dy;
+      const bool ok = nx >= 0 && nx < gh && ny >= 0 && ny < gw;
+      nb_idx[i] = ok ? nx * gw + ny : -1;
+      nb_coef[i] = ok ? grid_deg_inv_sqrt(x, y, gh, gw) * grid_deg_inv_sqrt(nx, ny, gh, gw) : 0.0f;
+    }
+    __syncthreads();
+    for (int64_t b = blockIdx.x; b < B; b += gridDim.x) {
+      const int64_t g0 = b * n;
+      for (int node = threadIdx.y; node < cn; node += blockDim.y) {
+        for (int c4 = threadIdx.x; c4 < H4; c4 += blockDim.x) {
+          float4 v[5], a[5];
 #pragma unroll
-        for (int k = 0; k < 5; ++k) {
-          const int j = nb_idx[node * 5 + k];
-          if (j < 0) continue;
-          const float coef = nb_coef[node * 5 + k];
-          const size_t off = (size_t)(g0 + j) * H4 + c4;
-          float4 v = in4[off];
-          if (BWD) {
-            const float4 a = act4[off];
-            v.x = a.x > 0.f ? v.x : 0.f; v.y = a.y > 0.f ? v.y : 0.f; v.z = a.z > 0.f ? v.z : 0.f; v.w = a.w > 0.f ? v.w : 0.f;
+          for (int k = 0; k < 5; ++k) {
+            const int j = nb_idx[node * 5 + k];
+            if (j < 0) continue;
+            const size_t off = (size_t)(g0 + j) * H4 + c4;
+            v[k] = in4[off];
+            if (BWD) a[k] = act4[off];
           }
-          acc.x = fmaf(coef, v.x, acc.x); acc.y = fmaf(coef, v.y, acc.y); acc.z = fmaf(coef, v.z, acc.z); acc.w = fmaf(coef, v.w, acc.w);
+          float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
+#pragma unroll
+          for (int k = 0; k < 5; ++k) {
+            if (nb_idx[node * 5 + k] < 0) continue;
+            if (BWD) {
+              v[k].x = a[k].x > 0.f ? v[k].x : 0.f; v[k].y = a[k].y > 0.f ? v[k].y : 0.f;
+              v[k].z = a[k].z > 0.f ? v[k].z : 0.f; v[k].w = a[k].w > 0.f ? v[k].w : 0.f;
+            }
+            const float coef = nb_coef[node * 5 + k];
+            acc.x = fmaf(coef, v[k].x, acc.x); acc.y = fmaf(coef, v[k].y, acc.y);
+            acc.z = fmaf(coef, v[k].z, acc.z); acc.w = fmaf(coef, v[k].w, acc.w);
+          }
+          if (!BWD) { acc.x = fmaxf(acc.x, 0.f); acc.y = fmaxf(acc.y, 0.f); acc.z = fmaxf(acc.z, 0.f); acc.w = fmaxf(acc.w, 0.f); }
+          out4[(size_t)(g0 + base + node) * H4 + c4] = acc;
         }
-        if (!BWD) { acc.x = fmaxf(acc.x, 0.f); acc.y = fmaxf(acc.y, 0.f); acc.z = fmaxf(acc.z, 0.f); acc.w = fmaxf(acc.w, 0.f); }
-        out4[(size_t)(g0 + node) * H4 + c4] = acc;
       }
     }
   }
@@ -1019,14 +1045,16 @@ int azg_graph_mean_relu_backward(const float* dout, const float* out, const int3
 }
 
 int azg_grid_aggregate_relu_forward(const float* sup, int64_t B, int gh, int gw, int H, float* out, azg_stream stream) {
-  AZG_REQUIRE(sup && out && gh >= 1 && gw >= 1 && H % 4 == 0, "azg_grid_aggregate_relu_forward: bad argument");
+  AZG_REQUIRE(sup && out && gh >= 1 && gw >= 1 && (int64_t)gh * gw <= GRID_AGG_MAX_NODES && H % 4 == 0,
+              "azg_grid_aggregate_relu_forward: bad argument");
   if (B <= 0) return AZG_OK;
   return launch_grid_aggregate<false>(sup, nullptr, B, gh, gw, H, out, (cudaStream_t)stream);
 }
 
 int azg_grid_aggregate_relu_backward(const float* dout, const float* out, int64_t B, int gh, int gw, int H, float* dsup,
                                      azg_stream stream) {
-  AZG_REQUIRE(dout && out && dsup && H % 4 == 0, "azg_grid_aggregate_relu_backward: bad argument");
+  AZG_REQUIRE(dout && out && dsup && gh >= 1 && gw >= 1 && (int64_t)gh * gw <= GRID_AGG_MAX_NODES && H % 4 == 0,
+              "azg_grid_aggregate_relu_backward: bad argument");
   if (B <= 0) return AZG_OK;
   return launch_grid_aggregate<true>(dout, out, B, gh, gw, H, dsup, (cudaStream_t)stream);
 }

@@ -212,8 +212,8 @@ int azg_graph_mean_relu_backward(const float* dout, const float* out, const int3
                                  float* dsup, azg_stream stream);
 /* Grid-graph layer of the roofline sweep (BASELINE configs[4]; SURVEY section 8d.5): relu(bmm(adj, sup)) with
  * adj = D^-1/2 (A + I) D^-1/2 of the gh x gw 4-neighbour grid (operator: FrozenLakeNet.GNNLayer,
- * FrozenLakeNet.py:8-33; normalisation: create_adjacency :68-72).  sup/out [B, gh*gw, H] fp32, H % 4 == 0.
- * backward: dsup = adj * (dout * (out > 0)). */
+ * FrozenLakeNet.py:8-33; normalisation: create_adjacency :68-72).  sup/out [B, gh*gw, H] fp32, H % 4 == 0,
+ * gh, gw >= 1, gh*gw <= 2^30.  backward: dsup = adj * (dout * (out > 0)). */
 int azg_grid_aggregate_relu_forward(const float* sup, int64_t B, int gh, int gw, int H, float* out, azg_stream stream);
 int azg_grid_aggregate_relu_backward(const float* dout, const float* out, int64_t B, int gh, int gw, int H,
                                      float* dsup, azg_stream stream);
@@ -223,7 +223,7 @@ int azg_grid_aggregate_relu_backward(const float* dout, const float* out, int64_
  *   forward:         out = relu(adj * (x W^T + b))                    x, out [B, gh*gw, H] fp32
  *   backward_input:  dx  = adj * ((dout * (out > 0)) W)
  * Weights are passed as operand images made by azg_grid_pack_weights (transpose = 1 for backward_input);
- * azg_grid_tc_supported: gh*gw <= 128 and H in {64, 128, 256}.  prec: AZG_PREC_BF16X3 or AZG_PREC_BF16. */
+ * azg_grid_tc_supported: gh*gw <= 256 and H in {64, 128, 256}.  prec: AZG_PREC_BF16X3 or AZG_PREC_BF16. */
 size_t azg_grid_packed_bytes(int H);
 int azg_grid_tc_supported(int gh, int gw, int H);
 int azg_grid_pack_weights(const float* w, int H, int transpose, void* packed, azg_stream stream);
