@@ -141,7 +141,7 @@ struct GridArgs {
   const float* act;    // BWD: the layer's output (ReLU gate), else null
   const uint8_t* w_hi; // weight image, k-block major: [KB][H rows x 64] (BWD: of W^T)
   const uint8_t* w_lo;
-  const float* bias;   // FWD: [H] or null
+  const float* bias;   // FWD: [H]; BWD: null (no bias term)
   float* out;
   int64_t B;           // graphs
   int gh, gw;
@@ -757,6 +757,9 @@ __global__ void reduce_cta_partials_kernel(const float* __restrict__ part, int c
   out[i] = s;
 }
 
+// most CTAs of one weight-gradient launch: azg_grid_dw_scratch_floats holds one [H, H] + [H] partial per CTA
+constexpr int DW_MAX_CTAS = 160;
+
 template <int H, bool X3>
 int launch_dw(const float* s, const float* x, int64_t rows, float* dw, float* db, float* scratch, cudaStream_t st) {
   static bool configured = false;
@@ -769,7 +772,8 @@ int launch_dw(const float* s, const float* x, int64_t rows, float* dw, float* db
     configured = true;
   }
   const int64_t kblocks = (rows + S::KR - 1) / S::KR;
-  const int grid = (int)(kblocks < sms ? kblocks : sms);
+  const int64_t ctas = sms < DW_MAX_CTAS ? sms : DW_MAX_CTAS;  // the kernel strides over the k-blocks by gridDim.x
+  const int grid = (int)(kblocks < ctas ? kblocks : ctas);
   DwArgs g{s, x, scratch, scratch + (size_t)grid * H * H, rows};
   grid_dw_tc_kernel<H, X3><<<grid, 512, S::TOTAL, st>>>(g);
   AZG_LAUNCH_CHECK();
@@ -835,8 +839,8 @@ extern "C" {
 size_t azg_grid_packed_bytes(int H) { return (size_t)H * H * 2 * 2; }  // hi image, lo image
 
 int azg_grid_tc_supported(int gh, int gw, int H) {
-  const int n = gh * gw;
-  return n >= 1 && n <= 256 && (H == 64 || H == 128 || H == 256);
+  // each side is checked before the product, so gh * gw can neither be negative nor wrap into range
+  return gh >= 1 && gw >= 1 && gh <= 256 && gw <= 256 && gh * gw <= 256 && (H == 64 || H == 128 || H == 256);
 }
 
 int azg_grid_pack_weights(const float* w, int H, int transpose, void* packed, azg_stream stream) {
@@ -851,7 +855,7 @@ int azg_grid_pack_weights(const float* w, int H, int transpose, void* packed, az
 
 int azg_grid_layer_tc_forward(const float* x, const void* packed_w, const float* bias, int64_t B, int gh, int gw, int H, int prec,
                               float* out, azg_stream stream) {
-  AZG_REQUIRE(x && packed_w && out, "azg_grid_layer_tc_forward: null pointer");
+  AZG_REQUIRE(x && packed_w && bias && out, "azg_grid_layer_tc_forward: null pointer");
   AZG_REQUIRE(azg_grid_tc_supported(gh, gw, H), "azg_grid_layer_tc_forward: unsupported shape %dx%d, H=%d", gh, gw, H);
   AZG_REQUIRE(prec == AZG_PREC_BF16X3 || prec == AZG_PREC_BF16, "azg_grid_layer_tc_forward: precision must be bf16x3 or bf16");
   if (B <= 0) return AZG_OK;
@@ -869,7 +873,7 @@ int azg_grid_layer_tc_backward_input(const float* dout, const float* act, const 
   return gridtc::dispatch<true>(g, H, prec, (cudaStream_t)stream);
 }
 
-size_t azg_grid_dw_scratch_floats(int H) { return (size_t)160 * ((size_t)H * H + H); }  // one partial per CTA (<= 160 SMs)
+size_t azg_grid_dw_scratch_floats(int H) { return (size_t)gridtc::DW_MAX_CTAS * ((size_t)H * H + H); }  // one partial per CTA
 
 int azg_grid_layer_tc_backward_weights(const float* s, const float* x, int64_t rows, int H, int prec, float* dw, float* db,
                                        float* scratch, azg_stream stream) {

@@ -91,7 +91,9 @@ class GridGNNStack(nn.Module):
 
     precision: "bf16x3" (default; fp32-level accuracy on the tensor cores), "bf16", or "fp32" (CUDA-core SGEMM +
     separate aggregation kernel -- also the path for graphs of more than 256 nodes or other hidden sizes).  Graphs of up to
-    128 nodes share 128-row tiles (128 // n graphs each), 129..256 nodes take one 256-row tile per graph.
+    128 nodes share 128-row tiles (128 // n graphs each), 129..256 nodes take one 256-row tile per graph.  The fused layer
+    takes gh, gw >= 1 with gh*gw <= 256 (azg_grid_tc_supported); tests/test_grid_tc_layer_gpu.py checks all of its kernels
+    against float64.
     The fp32 path takes any grid of up to 2^30 nodes and any hidden size divisible by 4; tests/test_grid_fp32_path_gpu.py
     checks it against float64 from 1 to 33,124 nodes and hidden 4 to 1,024."""
 

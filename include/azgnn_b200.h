@@ -223,7 +223,8 @@ int azg_grid_aggregate_relu_backward(const float* dout, const float* out, int64_
  *   forward:         out = relu(adj * (x W^T + b))                    x, out [B, gh*gw, H] fp32
  *   backward_input:  dx  = adj * ((dout * (out > 0)) W)
  * Weights are passed as operand images made by azg_grid_pack_weights (transpose = 1 for backward_input);
- * azg_grid_tc_supported: gh*gw <= 256 and H in {64, 128, 256}.  prec: AZG_PREC_BF16X3 or AZG_PREC_BF16. */
+ * azg_grid_tc_supported: gh, gw >= 1, gh*gw <= 256 and H in {64, 128, 256}; both layer entry points refuse any
+ * other shape.  bias [H] is required.  prec: AZG_PREC_BF16X3 or AZG_PREC_BF16. */
 size_t azg_grid_packed_bytes(int H);
 int azg_grid_tc_supported(int gh, int gw, int H);
 int azg_grid_pack_weights(const float* w, int H, int transpose, void* packed, azg_stream stream);

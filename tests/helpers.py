@@ -178,3 +178,24 @@ def assert_tables_equal(got, want, check_types=True):
             assert gq == q, ("Qsa", a, gq, q)  # bit-exact
             if check_types:
                 assert gt == t, ("Q type", a, gt, t)
+
+
+def grid_neighbours(gh, gw, device="cpu"):
+    """Neighbour table of the gh x gw grid in the kernel's order (self, up, down, left, right): idx [n, 5] int64 (-1 where
+    the neighbour is off the grid) and float64 coef [n, 5] = 1 / sqrt(d_i d_j), d = 1 + number of grid neighbours."""
+    node = torch.arange(gh * gw, device=device)
+    x, y = node // gw, node % gw
+    nx = x[:, None] + torch.tensor([0, -1, 1, 0, 0], device=device)
+    ny = y[:, None] + torch.tensor([0, 0, 0, -1, 1], device=device)
+    ok = (nx >= 0) & (nx < gh) & (ny >= 0) & (ny < gw)
+    deg = ok.sum(1).double()
+    idx = torch.where(ok, nx * gw + ny, -1)
+    coef = torch.where(ok, 1.0 / torch.sqrt(deg[:, None] * deg[idx.clamp(min=0)]), 0.0)
+    return idx, coef
+
+
+def aggregate64(v, idx, coef):
+    """adj v for v [B, n, H] float64, and the sum over k of |a_ik| |v_k| of every output"""
+    g = v[:, idx.clamp(min=0)]  # [B, n, 5, H]; absent neighbours have coefficient 0
+    c = coef[None, :, :, None]
+    return (g * c).sum(2), (g.abs() * c).sum(2)
