@@ -23,6 +23,8 @@ PACKED_AS = {PREC_F16F8_KS: PREC_F16F8, PREC_BF16X3_KS: PREC_BF16X3}  # precisio
 PRECISION_NAMES = {v: k for k, v in PRECISIONS.items()}
 TAG_NONE, TAG_F32, TAG_PYFLOAT, TAG_PYINT = -1, 0, 1, 2
 CELL_I8, CELL_I64, CELL_F32, CELL_F64 = 0, 1, 2, 3
+# search semantics of the arena (args.b200_search_semantics): the reference's backup, or Q negated before the update
+SEARCH_SEMANTICS = {"reference": 0, "alphazero": 1}
 
 _vp, _i, _i64, _sz, _d = C.c_void_p, C.c_int, C.c_int64, C.c_size_t, C.c_double
 
@@ -113,6 +115,7 @@ SIGNATURES = {
     "azg_arena_create": (_i, [C.POINTER(_vp), _i, _i, _i, _i, _i, _d, _vp, _sz, C.c_char_p, _vp]),
     "azg_arena_destroy": (_i, [_vp]),
     "azg_arena_copy_from": (_i, [_vp, _vp, _vp]),
+    "azg_arena_set_semantics": (_i, [_vp, _i]),
     "azg_arena_action_size": (_i, [_vp]),
     "azg_arena_reset": (_i, [_vp, _vp, _i, _vp]),
     "azg_arena_set_roots": (_i, [_vp, _vp, _vp]),

@@ -28,10 +28,20 @@ def default_capacity(kind, n, sims_per_move):
     return sims_per_move * plies + 16
 
 
+def semantics_code(name):
+    """`b200_search_semantics` value -> AZG_SEARCH_* (ValueError for anything but "reference" / "alphazero")"""
+    if not isinstance(name, str) or name not in _lib.SEARCH_SEMANTICS:
+        raise ValueError(f"b200_search_semantics must be one of {sorted(_lib.SEARCH_SEMANTICS)}, got {name!r}")
+    return _lib.SEARCH_SEMANTICS[name]
+
+
 class DeviceArena:
     def __init__(self, kind, n, n_games, sims_per_move, cpuct, capacity=None, max_depth=None, fl_map=None,
-                 device=None):
+                 device=None, semantics="reference"):
+        """semantics: backup of two-player searches, "reference" (MCTS.py:228-240) or "alphazero" (see set_semantics)"""
+        semantics_code(semantics)
         self._open(device)
+        self.semantics = semantics
         self._create_args = dict(kind=kind, n=n, sims_per_move=sims_per_move, cpuct=cpuct, fl_map=fl_map)
         self.kind, self.n, self.G = kind, n, int(n_games)
         self.A = action_size(kind, n)
@@ -70,7 +80,17 @@ class DeviceArena:
         handle = C.c_void_p()
         self._check(self.lib.azg_arena_create(C.byref(handle), GAME_KINDS[c["kind"]], c["n"], self.G, int(capacity), self.max_depth,
                                              float(c["cpuct"]), ptr(mem), nbytes, fl, self._stream()))
+        self._check(self.lib.azg_arena_set_semantics(handle, semantics_code(self.semantics)))
         return handle
+
+    def set_semantics(self, semantics):
+        """"alphazero": a two-player search stores into Qsa(s,a) the child's value negated, i.e. from the point of view
+        of the player who picks a at s, and PUCT maximises that player's value.  "reference": the reference's backup,
+        which stores the child's value before negating it.  Single-player games are the same in both.  Applies to the
+        searches queued after the call (a captured search graph keeps the mode it was captured with)."""
+        code = semantics_code(semantics)
+        self._check(self.lib.azg_arena_set_semantics(self.handle, code))
+        self.semantics = semantics
 
     def node_count(self, g=0):
         """entries in game g's table (synchronises)"""

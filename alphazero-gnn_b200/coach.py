@@ -22,7 +22,7 @@ from random import shuffle
 
 import numpy as np
 
-from .mcts import MCTS, arg
+from .mcts import MCTS, arg, example_symmetries, search_semantics
 from .selfplay import BatchedSelfPlay
 
 log = logging.getLogger(__name__)
@@ -97,6 +97,7 @@ class Coach:
     def __init__(self, game, nnet, args, arena_factory=None):
         self.game, self.nnet, self.args = game, nnet, args
         self._arena_factory = arena_factory  # tests inject the host check arena
+        self.symmetries = example_symmetries(game, search_semantics(args))
         self.pnet = None
         self.mcts = self._new_mcts(self.nnet)
         self.trainExamplesHistory = []
@@ -121,7 +122,7 @@ class Coach:
             canonicalBoard = self.game.getCanonicalForm(board, self.curPlayer)
             temp = int(episodeStep < arg(self.args, "tempThreshold"))
             pi = self.mcts.getActionProb(canonicalBoard, temp=temp)
-            sym = self.game.getSymmetries(canonicalBoard, pi)
+            sym = self.symmetries(canonicalBoard, pi)
             for b, p in sym:
                 trainExamples.append([b, self.curPlayer, p, None])
             if self._use_gnn():

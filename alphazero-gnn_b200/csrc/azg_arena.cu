@@ -209,7 +209,13 @@ int azg_arena_copy_from(azg_arena* dst, const azg_arena* src, azg_stream stream)
               "azg_arena_copy_from: the destination must be the same game with at least the source's capacity (%d < %d?)", d.cap, s.cap);
   arena_copy_kernel<<<d.G, 256, 0, (cudaStream_t)stream>>>(d, s);
   AZG_LAUNCH_CHECK();
+  dst->view.semantics = s.semantics;  // a grown table continues the search it holds
   return AZG_OK;
+}
+
+int azg_arena_set_semantics(azg_arena* a, int semantics) {
+  AZG_REQUIRE(a != nullptr, "azg_arena_set_semantics: null arena");
+  return azg_view_set_semantics(&a->view, semantics);
 }
 
 int azg_arena_set_roots(azg_arena* a, const uint64_t* states, azg_stream stream) {

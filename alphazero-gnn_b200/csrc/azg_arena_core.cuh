@@ -40,6 +40,7 @@ static inline float azg_fdiv(float a, float b) { volatile float r = a / b; retur
 struct AzgArenaView {
   AzgRules rules;
   int G, cap, hcap, max_depth, A, two_player;
+  int semantics;  // AZG_SEARCH_REFERENCE / AZG_SEARCH_ALPHAZERO, read by azg_backup only
   int p_f32;  // valid masks are int8 (FrozenLakeGame.py:125): Ps and the PUCT score stay float32 (NEP 50)
   double cpuct;
   // per game
@@ -186,10 +187,15 @@ AZG_HD float azg_np_sum_f32(const float* x, int n) {
   return azg_fadd(0.0f, res);
 }
 
-// lane 0: walk the recorded path back up, MCTS.py:228-240
+// lane 0: walk the recorded path back up, MCTS.py:228-240.  Two-player games negate v once per level after the edge
+// update.  In the AlphaZero semantics the negation comes before the update instead (Q from the point of view of the
+// player who picks the edge), which stores the same sequence as this walk started from -v.  The mode is a uniform
+// branch rather than a template parameter: it is the same for all games of a launch, costs one negation per backup,
+// and keeps one set of arena kernels for both modes.
 AZG_HD void azg_backup(const AzgArenaView& a, int g, int depth, AzgVal v) {
   const int32_t* pn = a.path_node + (size_t)g * a.max_depth;
   const int8_t* pa = a.path_act + (size_t)g * a.max_depth;
+  if (a.two_player && a.semantics == AZG_SEARCH_ALPHAZERO) v = azg_neg(v);
   for (int i = depth - 1; i >= 0; --i) {
     const size_t node = (size_t)g * a.cap + pn[i];
     const size_t e = node * a.A + pa[i];
@@ -425,6 +431,20 @@ AZG_HD void azg_advance_game(const AzgArenaView& a, int g, int action, double* e
   ended[g] = e.d;
   ended_tag[g] = (int8_t)e.tag;
 }
+
+// ---- search semantics: validated once, shared by the library and the host check build ---------------------------
+static inline int azg_view_set_semantics(AzgArenaView* v, int semantics) {
+  AZG_REQUIRE(semantics == AZG_SEARCH_REFERENCE || semantics == AZG_SEARCH_ALPHAZERO,
+              "azg_arena_set_semantics: unknown search semantics %d (0 = reference, 1 = alphazero)", semantics);
+  v->semantics = semantics;
+  return AZG_OK;
+}
+#if !defined(__CUDACC__)
+// The host check build (tests/hostcheck) compiles this file with a host compiler and binds every azg_arena_* entry
+// point of include/azgnn_b200.h under an `azgh_` name.  Its handle is a struct whose first and only member is the
+// view, so the handle points at the view.
+extern "C" int azgh_arena_set_semantics(AzgArenaView* a, int semantics) { return azg_view_set_semantics(a, semantics); }
+#endif
 
 // ---- table growth: copy game g from `s` into the larger `d` (same game, A, max_depth; d.cap >= s.cap) ------------
 // part 1 (any number of lanes): clear d's hash slots and copy the node and edge arrays verbatim (node indices are kept)

@@ -50,8 +50,11 @@ class _TwoPlayerGame:
 class Connect4Game(_TwoPlayerGame):
     azg_kind = "connect4"
 
-    def __init__(self, board_size=7):
+    def __init__(self, board_size=7, mirror_columns=False):
+        """mirror_columns: getSymmetries mirrors the board over its columns, as it mirrors pi (the AlphaZero search
+        semantics, b200_search_semantics = "alphazero"); False keeps the reference's method"""
         self.board_size = board_size
+        self.mirror_columns = mirror_columns
 
     def getInitBoard(self):
         return np.zeros((self.board_size, self.board_size), dtype=np.int64)
@@ -87,11 +90,13 @@ class Connect4Game(_TwoPlayerGame):
 
     def getSymmetries(self, board, pi):
         """Connect4Game.py:189-215 -- note the reference mirrors the board with np.fliplr (the row
-        axis of a [column][row] board) while mirroring pi over columns; kept as is."""
+        axis of a [column][row] board, which turns it upside down) while mirroring pi over columns; kept
+        as is unless mirror_columns, which reverses the columns instead (board[::-1, :])."""
         assert len(pi) == self.board_size + 1
         mpi = np.copy(pi)
         mpi[:self.board_size] = np.asarray(pi)[:self.board_size][::-1]
-        return [(board, pi), (np.fliplr(board), mpi)]
+        mirrored = np.flipud(board) if self.mirror_columns else np.fliplr(board)
+        return [(board, pi), (mirrored, mpi)]
 
 
 class TicTacToeGame(_TwoPlayerGame):

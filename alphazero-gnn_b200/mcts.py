@@ -15,7 +15,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from .arena import DeviceArena, action_size
+from .arena import DeviceArena, action_size, semantics_code
 
 EPS = 1e-8  # MCTS.py:6
 
@@ -29,6 +29,22 @@ def arg(args, name, default=None):
             return args[name]
         except (KeyError, TypeError, IndexError):
             return default
+
+
+def search_semantics(args):
+    """args.b200_search_semantics: "reference" (default) or "alphazero"; any other value raises ValueError"""
+    sem = arg(args, "b200_search_semantics", "reference")
+    semantics_code(sem)
+    return sem
+
+
+def example_symmetries(game, semantics):
+    """The symmetric forms self-play turns each position into: the game's own `getSymmetries`, except for Connect4 in
+    the "alphazero" semantics, whose mirror reverses the columns (games.Connect4Game(mirror_columns=True))."""
+    if semantics == "alphazero" and game_kind(game) == "connect4":
+        from .games import Connect4Game
+        return Connect4Game(game.getBoardSize()[0], mirror_columns=True).getSymmetries
+    return game.getSymmetries
 
 
 def game_kind(game):
@@ -137,11 +153,14 @@ class BatchedMCTS:
         assert self.A == action_size(self.kind, self.n)
         self.G = n_games
         self.use_gnn = bool(arg(args, "use_gnn", False))
+        self.semantics = search_semantics(args)
         sims = int(arg(args, "numMCTSSims")) + (int(arg(args, "expand_by", 5)) if self.use_gnn else 0)
         if arena is None:
             fl_map = b"".join(np.asarray(game.desc).reshape(-1).tolist()) if self.kind == "frozenlake" else None
             arena = DeviceArena(self.kind, self.n, n_games, sims, float(arg(args, "cpuct")), capacity=capacity,
-                                max_depth=max_depth, fl_map=fl_map)
+                                max_depth=max_depth, fl_map=fl_map, semantics=self.semantics)
+        elif arena.semantics != self.semantics:
+            arena.set_semantics(self.semantics)  # the search settings decide, as for cpuct and numMCTSSims
         self.arena = arena
         self.device_eval = hasattr(nnet, "forward_states")
         # compacted leaf batches (only waiting games are evaluated; the count never leaves the device)

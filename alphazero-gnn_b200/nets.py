@@ -22,7 +22,7 @@ import torch
 
 from . import _lib, modules
 from ._lib import ptr, stream
-from .mcts import arg, game_kind, pack_states
+from .mcts import arg, game_kind, pack_states, search_semantics
 
 _CELL = {torch.int8: _lib.CELL_I8, torch.int64: _lib.CELL_I64, torch.float32: _lib.CELL_F32,
          torch.float64: _lib.CELL_F64}
@@ -40,6 +40,7 @@ class _Base:
     kind = None
 
     def _common(self, game, args):
+        search_semantics(args)  # a bad b200_search_semantics fails here, not at the first search
         self.board_x, self.board_y = game.getBoardSize()
         assert self.board_x == self.board_y, "square boards only (Connect4Game.py:123-137)"
         self.n = self.board_x

@@ -19,21 +19,37 @@ rules (success beats failure, fewer steps to succeed, more steps survived before
 """
 import numpy as np
 
+from .arena import semantics_code
 from .mcts import BatchedMCTS, arg, pack_states
 
 
+def with_args(args, **kv):
+    """a copy of a config (dict, dotdict or namespace) with some keys replaced"""
+    a = type(args)(args) if isinstance(args, dict) else dict(vars(args))
+    a.update(kv)
+    return a if isinstance(args, dict) else type("Args", (), a)()
+
+
 class BatchedArena:
-    def __init__(self, game, nnet1, nnet2, args, arena_factory=None, args2=None):
-        """args2: search settings of player 2 when they differ from player 1's (e.g. use_gnn, main.py:96-103)"""
+    def __init__(self, game, nnet1, nnet2, args, arena_factory=None, args2=None, semantics=None):
+        """args2: search settings of player 2 when they differ from player 1's (e.g. use_gnn, main.py:96-103).
+        semantics: (player 1's, player 2's) b200_search_semantics, replacing the configs' own -- e.g. the same network
+        searching with "alphazero" against "reference" backups."""
         assert getattr(game, "is_two_player", True), "BatchedArena pits two-player games"
         self.game, self.nets = game, (nnet1, nnet2)
         self.args = (args, args if args2 is None else args2)
+        if semantics is not None:
+            for s in semantics:
+                semantics_code(s)  # ValueError now rather than at the first game
+            self.args = tuple(with_args(a, b200_search_semantics=s) for a, s in zip(self.args, semantics))
+        self._per_side = semantics is not None
         self._arena_factory = arena_factory
         self.graph_search = bool(arg(args, "b200_graph_search", False))  # measured: no gain for one playGames call (capture costs what replay saves)
 
-    def _mcts(self, net, n_games):
+    def _mcts(self, k, n_games):
         arena = self._arena_factory(n_games) if self._arena_factory else None
-        a = self.args[self.nets.index(net)] if self.nets[0] is not self.nets[1] else self.args[0]
+        net = self.nets[k]
+        a = self.args[k] if self._per_side or self.nets[0] is not self.nets[1] else self.args[0]
         sims = int(arg(a, "numMCTSSims"))
         n = self.game.getBoardSize()[0]
         # a game's tree lives for the whole game: every simulation of every ply it is searched on adds <= 1 entry
@@ -46,7 +62,7 @@ class BatchedArena:
             return 0, 0, 0
         g = self.game
         # group 0: net 0 is player +1 (moves first); group 1: net 1 is player +1
-        mcts = [[self._mcts(self.nets[k], half) for _grp in range(2)] for k in range(2)]
+        mcts = [[self._mcts(k, half) for _grp in range(2)] for k in range(2)]
         # Positions live in the arenas as packed canonical states: a ply is set_roots -> numMCTSSims lock-step searches ->
         # arg-max of the visit counts -> `advance` (the arena's own rules play the move and report getGameEnded for the
         # player to move), with no per-game Python game logic (100 games x ~40 plies of it took 0.5 s of a 0.77 s arena)
@@ -157,9 +173,6 @@ class BatchedSinglePlayerArena:
 def pit_gnn_vs_regular(game, gnn_nnet, reg_nnet, config_args, num=None):
     """main.py:60-138 (`--pit_gnn`): the GNN-enhanced model (searching with predict_with_gnn) against the regular
     model (predict), `arenaCompare` games, all in flight.  Returns (gnn_wins, reg_wins, draws)."""
-    def with_gnn(flag):
-        a = type(config_args)(config_args) if isinstance(config_args, dict) else dict(vars(config_args))
-        a["use_gnn"] = flag
-        return a if isinstance(config_args, dict) else type("Args", (), a)()
     num = arg(config_args, "arenaCompare") if num is None else num
-    return BatchedArena(game, gnn_nnet, reg_nnet, with_gnn(True), args2=with_gnn(False)).playGames(num)
+    return BatchedArena(game, gnn_nnet, reg_nnet, with_args(config_args, use_gnn=True),
+                        args2=with_args(config_args, use_gnn=False)).playGames(num)

@@ -26,12 +26,13 @@ from .mcts import game_kind, pack_states, typed_value, unpack_state
 _I8 = torch.int8
 
 
-def symmetry_tables(game):
-    """(board_perm [S, n*n] int32, pi_perm [S, A] int32): output cell d of symmetry s shows input cell board_perm[s, d]"""
+def symmetry_tables(game, symmetries=None):
+    """(board_perm [S, n*n] int32, pi_perm [S, A] int32): output cell d of symmetry s shows input cell board_perm[s, d].
+    symmetries: the (board, pi) -> forms function to tabulate, default game.getSymmetries"""
     n = game.getBoardSize()[0]
     A = game.getActionSize()
     idx_board = np.arange(n * n, dtype=np.int64).reshape(n, n)
-    forms = game.getSymmetries(idx_board, list(range(A)))
+    forms = (symmetries or game.getSymmetries)(idx_board, list(range(A)))
     bp = np.stack([np.asarray(b, dtype=np.int64).reshape(-1) for b, _ in forms]).astype(np.int32)
     pp = np.stack([np.asarray(p, dtype=np.int64).reshape(-1) for _, p in forms]).astype(np.int32)
     return bp, pp
@@ -167,9 +168,9 @@ class DeviceExamples(_Columns):
     COLS = (("states", torch.int64, False), ("pi", torch.float64, True), ("v", torch.float64, False), ("vtag", _I8, False),
             ("sym", _I8, False))
 
-    def __init__(self, game, device=None):
+    def __init__(self, game, device=None, symmetries=None):
         self._init_columns(game, device)
-        bp, pp = symmetry_tables(game)
+        bp, pp = symmetry_tables(game, symmetries)
         self.S = bp.shape[0]
         self._bp = torch.from_numpy(bp).to(self.device)
         self._pp = torch.from_numpy(pp).to(self.device)

@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from ._lib import ptr
-from .mcts import BatchedMCTS, arg, pack_states
+from .mcts import BatchedMCTS, arg, example_symmetries, pack_states
 
 EPS = 1e-8
 
@@ -90,6 +90,7 @@ class BatchedSelfPlay:
         self.use_gnn = bool(arg(args, "use_gnn", False))
         self.mcts = BatchedMCTS(game, nnet, args, n_games=self.G, arena=arena)
         self.kind, self.n, self.A = self.mcts.kind, self.mcts.n, self.mcts.A
+        self.symmetries = example_symmetries(game, self.mcts.semantics)
         self.rng = np.random.default_rng(seed)
         # collect_examples: False (throughput runs), True (host lists, the reference's tuples), or "device": standard
         # examples are assembled on the GPU (replay.DeviceExamples: history in HBM, symmetries + value signing in one
@@ -118,7 +119,7 @@ class BatchedSelfPlay:
             self.h_player = torch.zeros(self.t_cap, self.G, dtype=torch.int32, device=dev)
             self.h_int = torch.zeros(self.t_cap, self.G, dtype=torch.int8, device=dev)
             self.h_player_host = np.zeros((self.t_cap, self.G), dtype=np.int32)
-            self.device_examples = DeviceExamples(game, dev)
+            self.device_examples = DeviceExamples(game, dev, symmetries=self.symmetries)
             self.device_gnn_examples = DeviceGnnExamples(game, dev)
             if reserve_episodes:  # an episode stores at most t_cap positions, each in S symmetric forms
                 self.device_examples.reserve(int(reserve_episodes) * self.t_cap * self.device_examples.S)
@@ -179,7 +180,7 @@ class BatchedSelfPlay:
         std, gnn = [], []
         for board, pl, pi, rec in self.history[g]:
             sign = r * ((-1) ** (pl != cur))
-            sym = self.game.getSymmetries(board, pi)
+            sym = self.symmetries(board, pi)
             for b, p in sym:
                 std.append((b, p, sign))
             if rec is not None:

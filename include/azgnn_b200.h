@@ -323,8 +323,17 @@ int azg_arena_destroy(azg_arena* a);
 /* Table growth: the reference's dicts are unbounded (MCTS.py:15-21) and Coach / Arena reuse one MCTS object across all
  * arenaCompare games (Coach.py:128-142), so a table can outgrow any fixed capacity.  Copies every game of `src` (nodes,
  * edges, per-game search state) into `dst`, an arena of the same game / n_games / max_depth created with a larger
- * capacity_nodes, and rebuilds the hash for the new size; node indices are preserved. */
+ * capacity_nodes, and rebuilds the hash for the new size; node indices are preserved.  `dst` takes `src`'s search
+ * semantics. */
 int azg_arena_copy_from(azg_arena* dst, const azg_arena* src, azg_stream stream);
+/* Backup semantics of a two-player search (single-player games are unaffected).  AZG_SEARCH_REFERENCE (the default
+ * of a new arena): Qsa(s,a) holds the child's value before it is negated (MCTS.py:228-240), i.e. from the point of
+ * view of the player to move at the child.  AZG_SEARCH_ALPHAZERO: the value is negated first, so Qsa(s,a) is held
+ * from the point of view of the player to move at s, the one who picks a.  Takes effect from the next launch;
+ * any other value is refused with AZG_ERR_INVALID. */
+#define AZG_SEARCH_REFERENCE 0
+#define AZG_SEARCH_ALPHAZERO 1
+int azg_arena_set_semantics(azg_arena* a, int semantics);
 int azg_arena_action_size(const azg_arena* a);
 /* new MCTS object for the listed games (Coach.py:96): clear their tables.  game_ids: device
  * int32 [count], or NULL = all games. */
