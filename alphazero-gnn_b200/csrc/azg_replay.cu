@@ -101,7 +101,8 @@ __global__ void gather_examples_kernel(const State2* __restrict__ states, const 
 //   expand_tree record     initial / expanded visit policies and the expanded value sum_a Q N / sum_a N with the NEP-50
 //                          promotion order of the reference's scalar loop (Python number until the first np.float32 term)
 // Every rounding is spelled out (no FMA contraction): the results equal selfplay.probs_from_counts / sample_actions and
-// mcts.expanded_values bit for bit, which tests/test_replay_gpu.py checks through whole self-play runs.
+// mcts.expanded_values bit for bit, which tests/test_selfplay_move_gpu.py checks through the C ABI and
+// tests/test_replay_gpu.py through whole self-play runs.
 constexpr int MOVE_MAX_A = 65;  // TicTacToe 8x8 + pass (MOVE_MAX_A of the arena core)
 __global__ void __launch_bounds__(128) selfplay_move_kernel(azg_move_params p) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
@@ -109,6 +110,11 @@ __global__ void __launch_bounds__(128) selfplay_move_kernel(azg_move_params p) {
   const int A = p.A;
   const int t = p.slot[g];
   if (t < 0) {
+    p.actions[g] = -1;
+    return;
+  }
+  if (t >= p.T && (p.h_states || (p.n1 && p.rec_ip))) {  // no history row to write into: an error, nothing is written
+    atomicOr(p.flags, 2);
     p.actions[g] = -1;
     return;
   }
@@ -219,7 +225,8 @@ int azg_selfplay_move(const azg_move_params* p, azg_stream stream) {
   AZG_REQUIRE(p && p->G > 0 && p->A >= 1 && p->A <= MOVE_MAX_A, "azg_selfplay_move: bad sizes");
   AZG_REQUIRE(p->n0 && p->greedy && p->u_tie && p->u_sample && p->slot && p->actions && p->flags, "azg_selfplay_move: null pointer");
   AZG_REQUIRE(!p->h_states || (p->roots && p->player && p->h_pi && p->h_player && p->h_int && p->T > 0), "azg_selfplay_move: history buffers missing");
-  AZG_REQUIRE(!p->n1 || !p->rec_ip || (p->q1 && p->t1 && p->v0 && p->rec_iv && p->rec_ep && p->rec_ev && p->rec_evtag), "azg_selfplay_move: record buffers missing");
+  AZG_REQUIRE(!p->n1 || !p->rec_ip || (p->q1 && p->t1 && p->v0 && p->rec_iv && p->rec_ep && p->rec_ev && p->rec_evtag && p->T > 0),
+              "azg_selfplay_move: record buffers missing");
   selfplay_move_kernel<<<grid_for(p->G, 128), 128, 0, (cudaStream_t)stream>>>(*p);
   AZG_LAUNCH_CHECK();
   return AZG_OK;

@@ -361,8 +361,11 @@ class BatchedSelfPlay:
         # ---- the one synchronisation of the move ----
         e_val, e_tag = ar.to_host(e_dev), ar.to_host(tag_dev)
         ar.check_status()
-        if int(self._flags.item()):
+        flags = int(self._flags.item())
+        if flags & 1:
             raise RuntimeError("self-play: a game had no root visits after its searches")
+        if flags & 2:
+            raise RuntimeError(f"self-play: a history slot is past the {p.T} slots per game")
         self.moves_played += int(self.active.sum())
         if self.two_player:
             self.player = -self.player

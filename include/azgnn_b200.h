@@ -252,7 +252,9 @@ int azg_grid_layer_tc_backward_weights(const float* s, const float* x, int64_t r
  * temp-0 tie-break from u_tie), np.random.choice (inverse CDF at u_sample), the history slot [t, g] (root state, policy, player,
  * temp-0 flag) and, with n1 / q1 / t1 / v0, expand_tree's record (MCTS.py:94-143: initial / expanded visit policies, expanded
  * value with the NEP-50 promotion order).  The uniforms come from the caller's NumPy stream, so the results equal the host
- * path's bit for bit.  slot[g] < 0 skips the game (actions[g] = -1).  flags bit 0: a game had no root visits. */
+ * path's bit for bit.  slot[g] < 0 skips the game (actions[g] = -1).  flags bit 0: a game had no root visits.
+ * flags bit 1: with history or record buffers, a game's slot[g] >= T; that game gets actions[g] = -1 and no row is written.
+ * Record buffers need T > 0 as history buffers do. */
 typedef struct azg_move_params {
   int G, A, T;              /* games, actions, history slots per game */
   const int32_t* n0;        /* [G,A] root visit counts after the numMCTSSims searches */

@@ -180,9 +180,12 @@ def case_rules(rules_eval, tag):
     """valid masks, terminal values (+types) and canonical successor states vs the reference."""
     g = golden("rules_" + tag)
     name, game, n = _mk_game(tag)
+    _check_rules(rules_eval, name, game, n, g["canonical"])
+
+
+def _check_rules(rules_eval, name, game, n, canon):
     A = game.getActionSize()
     fl_map = b"".join(game.desc.reshape(-1).tolist()) if name == "frozenlake" else None
-    canon = g["canonical"]
     states = pack_states(name, canon)
     valids, ended, etag, nxt = rules_eval(name, n, fl_map, states)
     for i in range(canon.shape[0]):
@@ -201,6 +204,163 @@ def case_rules(rules_eval, tag):
                     nb, npl = game.getNextState(np.array(b, copy=True), 1, a)
                     want = pack_states(name, np.asarray(game.getCanonicalForm(nb, npl))[None])[0]
                     assert np.array_equal(nxt[i, a], want), (i, a)
+
+
+def _win_lines(name, n):
+    """every winning line as a list of (x, y) cells: Connect4 runs of min(4, n) in four directions (Board.is_win),
+    TicTacToe full rows, columns and both diagonals"""
+    if name == "tictactoe":
+        return ([[(x, y) for x in range(n)] for y in range(n)] + [[(x, y) for y in range(n)] for x in range(n)] +
+                [[(i, i) for i in range(n)], [(i, n - 1 - i) for i in range(n)]])
+    k = min(4, n)
+    lines = []
+    for dx, dy in ((1, 0), (0, 1), (1, 1), (1, -1)):
+        for x in range(n):
+            for y in range(n):
+                cells = [(x + i * dx, y + i * dy) for i in range(k)]
+                if all(0 <= cx < n and 0 <= cy < n for cx, cy in cells):
+                    lines.append(cells)
+    return lines
+
+
+def _without_lines(game, board, lines, fixed, rng, tries=4000):
+    """min-conflicts repair: flip free stones that sit on a one-colour line until neither side has a line (or None)"""
+    b = board.copy()
+    for _ in range(tries):
+        bad = [c for line in lines for c in line
+               if c not in fixed and abs(int(sum(b[x, y] for x, y in line))) == len(line)]
+        if not bad:
+            return b
+        x, y = bad[int(rng.integers(len(bad)))]
+        b[x, y] = -b[x, y]
+    return None
+
+
+def _edge_positions(name, game, n, rng):
+    """built positions at the edges of the rules: a line of either colour through each corner in every direction that
+    passes one (cell 0, cell n*n - 1 = bit 63 at 8x8, and the anti-diagonal corners), full-board draws where only
+    the pass move is valid, and boards whose one empty cell wins for the player to move"""
+    lines = _win_lines(name, n)
+    corners = {(0, 0), (n - 1, n - 1), (0, n - 1), (n - 1, 0)}
+    out = []
+    for line in lines:
+        if corners & set(line):
+            for colour in (1, -1):
+                b = np.zeros((n, n), dtype=np.int64)
+                for x, y in line:
+                    b[x, y] = colour
+                out.append(b)
+    draws, last = 0, 0
+    for _ in range(12):
+        full = _without_lines(game, rng.choice([1, -1], size=(n, n)).astype(np.int64), lines, set(), rng)
+        if full is None:
+            continue
+        assert game.getGameEnded(full, 1) == 1e-4 and list(game.getValidMoves(full, 1)).count(1) == 1
+        out.append(full)
+        draws += 1
+        line = lines[int(rng.integers(len(lines)))]
+        z = line[int(rng.integers(len(line)))]
+        b = full.copy()
+        for x, y in line:
+            b[x, y] = 1
+        b[z] = 0
+        b = _without_lines(game, b, lines, set(line), rng)
+        if b is None or game.getGameEnded(b, 1) != 0:
+            continue
+        if name == "connect4":
+            a = z[0]
+        else:
+            a = z[0] * n + z[1]
+        nb, npl = game.getNextState(b.copy(), 1, a)
+        if game.getGameEnded(nb, 1) == 1:
+            out.append(b)
+            out.append(game.getCanonicalForm(nb, npl))
+            last += 1
+    return out, draws, last
+
+
+def case_rules_playouts(rules_eval, kind, n, games=40, seed=0):
+    """`case_rules` on positions from random games played to the end with oracle.rules (every position of every game,
+    terminal ones included) and on built edge positions; FrozenLake: every cell of the map"""
+    name, game, _ = _mk_game(f"{kind}_{n}")
+    rng = np.random.default_rng(seed * 100 + n)
+    if name == "frozenlake":
+        canon = np.zeros((n * n, n, n))
+        canon.reshape(n * n, -1)[np.arange(n * n), np.arange(n * n)] = 1
+        _check_rules(rules_eval, name, game, n, canon)
+        return
+    pos = []
+    for _ in range(games):
+        board, player = game.getInitBoard(), 1
+        while True:
+            pos.append(game.getCanonicalForm(board, player))
+            if game.getGameEnded(board, player) != 0:
+                break
+            a = int(rng.choice(np.flatnonzero(game.getValidMoves(board, player))))
+            board, player = game.getNextState(board, player, a)
+    edges, draws, last = _edge_positions(name, game, n, rng)
+    if n >= 3:  # a 2x2 board always holds a line of two when full (every pair of its cells is a line)
+        assert draws > 0 and last > 0, (draws, last)
+    _check_rules(rules_eval, name, game, n, np.stack(pos + edges))
+
+
+RULES_REFUSED = [("tictactoe", 6), ("tictactoe", 7), ("tictactoe", 8)] + [(k, n) for k in ("connect4", "tictactoe") for n in (1, 9)]
+
+
+def case_refused_sizes(lib, make_arena, device, stream):
+    """Board sizes the rules do not accept: azg_rules_eval, azg_arena_bytes and azg_arena_create refuse them, and so
+    does the arena's Python handle"""
+    import ctypes as C
+    import pytest
+    import torch
+    from azgnn_b200.arena import GAME_KINDS
+    s = torch.zeros(1, 2, dtype=torch.int64, device=device)
+    valids = torch.zeros(1, dtype=torch.int32, device=device)
+    ended = torch.zeros(1, dtype=torch.float64, device=device)
+    etag = torch.zeros(1, dtype=torch.int8, device=device)
+    nxt = torch.zeros(1, 128, 2, dtype=torch.int64, device=device)
+    mem = torch.zeros(1 << 20, dtype=torch.uint8, device=device)
+    for kind, n in RULES_REFUSED:
+        game = GAME_KINDS[kind]
+        rc = lib.azg_rules_eval(game, n, None, s.data_ptr(), 1, valids.data_ptr(), ended.data_ptr(), etag.data_ptr(),
+                                nxt.data_ptr(), stream)
+        assert rc != 0, (kind, n)
+        assert lib.azg_arena_bytes(game, n, 1, 64, 8) == 0, (kind, n)
+        h = C.c_void_p()
+        rc = lib.azg_arena_create(C.byref(h), game, n, 1, 64, 8, 1.0, mem.data_ptr(), mem.numel(), None, stream)
+        assert rc != 0 and not h.value, (kind, n)
+        with pytest.raises(RuntimeError, match="unsupported arena configuration"):
+            make_arena(kind, n, 1, 4, 1.0)
+
+
+def case_uniform_prior_ties(make_arena, tag, roots=4, sims=80):
+    """A uniform-prior, zero-value net (as in case_known_answer) searched from a few roots at once against OracleMCTS:
+    early simulations tie exactly on every unvisited action, across the lanes of the CUDA arena's arg-max and among the
+    actions one lane holds, so the tables are equal only if ties go to the lowest action index everywhere."""
+    name, game, n = _mk_game(tag)
+    A = game.getActionSize()
+
+    class Uniform:
+        def predict(self, b):
+            return np.full(A, 1.0 / A, dtype=np.float32), np.float32(0.0)
+        predict_with_gnn = predict
+    args = dotdict(dict(numMCTSSims=sims, cpuct=1.0, use_gnn=False))
+    rng = np.random.default_rng(A)
+    boards = [game.getInitBoard()]
+    while len(boards) < roots:
+        b, player = game.getInitBoard(), 1
+        for _ in range(int(rng.integers(1, n))):
+            b, player = game.getNextState(b, player, int(rng.choice(np.flatnonzero(game.getValidMoves(b, player)))))
+        if game.getGameEnded(b, player) == 0:
+            boards.append(game.getCanonicalForm(b, player))
+    arena = make_arena(name, n, roots, sims, 1.0, capacity=2 * sims + 64)
+    bm = BatchedMCTS(game, Uniform(), args, n_games=roots, arena=arena)
+    bm.set_root_boards(boards)
+    pis = bm.getActionProbs(temp=1)
+    for g, root in enumerate(boards):
+        o = OracleMCTS(game, Uniform(), args)
+        assert np.array_equal(np.asarray(o.getActionProb(root, temp=1)), np.asarray(pis[g])), g
+        assert_tables_equal(mcts_as_tables(_View(bm.tables(g)), n, A), mcts_as_tables(o, n, A))
 
 
 def case_capacity_overflow(make_arena):

@@ -41,7 +41,7 @@ def test_known_answer():
     cases.case_known_answer(make_arena)
 
 
-@pytest.mark.parametrize("tag", ["c4_7", "ttt_4"])
+@pytest.mark.parametrize("tag", ["c4_7", "ttt_4", "c4_3", "c4_6", "c4_8", "ttt_5"])
 def test_lockstep_games(tag):
     cases.case_lockstep_games(make_arena, tag)
 
@@ -60,9 +60,24 @@ def test_capacity_overflow():
     cases.case_capacity_overflow(make_arena)
 
 
-@pytest.mark.parametrize("tag", ["c4_7", "ttt_3"])
+@pytest.mark.parametrize("tag", ["c4_7", "ttt_3", "c4_3", "c4_6", "c4_8", "ttt_5"])
 def test_compacted_leaf_batches(tag):
     cases.case_compact_lockstep(make_arena, tag)
+
+
+@pytest.mark.parametrize("kind,n", [("c4", n) for n in range(2, 9)] + [("ttt", n) for n in range(2, 6)] + [("fl", 4), ("fl", 8)])
+def test_rules_playouts(kind, n):
+    """every accepted board size: Connect4 8x8 is the only one that uses bit 63, TicTacToe 5x5 the only one with 26 actions"""
+    cases.case_rules_playouts(rules_eval, kind, n)
+
+
+def test_refused_board_sizes():
+    cases.case_refused_sizes(hostlib(), make_arena, "cpu", None)
+
+
+@pytest.mark.parametrize("tag", ["ttt_5", "c4_8"])
+def test_uniform_prior_ties(tag):
+    cases.case_uniform_prior_ties(make_arena, tag)
 
 
 def test_np_sum_order_matches_numpy():

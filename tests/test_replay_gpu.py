@@ -31,7 +31,8 @@ def _random_history(game, kind, n, E, rng):
     return boards, pis, players
 
 
-@pytest.mark.parametrize("kind,n", [("c4", 7), ("c4", 5), ("ttt", 3), ("ttt", 4), ("fl", 4), ("fl", 8)])
+@pytest.mark.parametrize("kind,n", [("c4", 7), ("c4", 5), ("ttt", 3), ("ttt", 4), ("fl", 4), ("fl", 8), ("c4", 8), ("c4", 6),
+                                    ("ttt", 5)])
 def test_emit_matches_host_symmetries_and_signs(kind, n):
     game = _game(kind, n)
     rng = np.random.default_rng(n)
@@ -61,7 +62,7 @@ def test_emit_matches_host_symmetries_and_signs(kind, n):
         assert gv == wv and type(gv) is type(wv)
 
 
-@pytest.mark.parametrize("kind,n", [("c4", 7), ("ttt", 4), ("fl", 4)])
+@pytest.mark.parametrize("kind,n", [("c4", 7), ("ttt", 4), ("fl", 4), ("c4", 8), ("ttt", 5)])
 def test_sample_equals_host_minibatch_and_round_trips(kind, n):
     game = _game(kind, n)
     rng = np.random.default_rng(1)
@@ -93,29 +94,50 @@ def test_sample_equals_host_minibatch_and_round_trips(kind, n):
 
 def test_device_collection_equals_host_collection():
     """Same seeds, same network: the examples gathered in HBM equal the host tuples (order included)."""
-    from azgnn_b200.nets import B200Connect4GNNWrapper
+    _check_device_collection("c4_5", sims=6, temp_threshold=4)
+
+
+@pytest.mark.parametrize("tag,sims,temp_threshold", [("ttt_4", 5, 4), ("ttt_5", 5, 6), ("c4_8", 4, 8), ("fl_4", 6, 4)])
+def test_device_collection_equals_host_collection_at_more_sizes(tag, sims, temp_threshold):
+    """TicTacToe 5x5 (26 actions) and Connect4 8x8 (bit 63 of the packed states), TicTacToe 4x4, and FrozenLake 4x4 with
+    the step cap that single-player device collection needs"""
+    _check_device_collection(tag, sims, temp_threshold)
+
+
+def _check_device_collection(tag, sims, temp_threshold):
+    """Same seeds, same network: the examples gathered in HBM (azg_selfplay_move tail, azg_emit_examples) equal the host
+    tuples, order and GNN records included.  Few simulations leave visit-count ties; moves before tempThreshold are
+    sampled at temperature 1, later ones greedily."""
+    from azgnn_b200.nets import B200Connect4GNNWrapper, B200FrozenLakeNet, B200TicTacToeGNNWrapper
     from azgnn_b200.selfplay import BatchedSelfPlay
-    game = games.Connect4Game(5)
-    args = dotdict(dict(lr=1e-3, dropout=0.3, epochs=2, batch_size=16, gnn_layers=2, use_gnn=True, numMCTSSims=6, cpuct=1.0,
-                        expand_by=3, tempThreshold=4, b200_precision="fp32"))
+    kind, n = tag.split("_")[0], int(tag.split("_")[1])
+    game = _game(kind, n)
+    use_gnn = kind != "fl"  # the FrozenLake network has no GNN head, so its episodes have no records
+    args = dotdict(dict(lr=1e-3, dropout=0.3, epochs=2, batch_size=16, gnn_layers=2, use_gnn=use_gnn, numMCTSSims=sims,
+                        cpuct=1.0, expand_by=3, tempThreshold=temp_threshold, b200_precision="fp32"))
     torch.manual_seed(0)
-    net = B200Connect4GNNWrapper(game, args)
+    net = {"c4": B200Connect4GNNWrapper, "ttt": B200TicTacToeGNNWrapper, "fl": B200FrozenLakeNet}[kind](game, args)
+    cap = 12 if kind == "fl" else None  # device collection of single-player episodes needs a step cap
     runs = {}
     for mode in (True, "device"):
-        sp = BatchedSelfPlay(game, net, args, 24, seed=5, collect_examples=mode)
+        sp = BatchedSelfPlay(game, net, args, 24, seed=5, collect_examples=mode, max_episode_steps=cap)
         fin = sp.play(40)
         runs[mode] = (sp, fin)
+    assert runs["device"][0].device_tail
     host_std = [e for std, _ in runs[True][1] for e in std]
     host_gnn = [e for _, gnn in runs[True][1] for e in gnn]
+    greedy = [np.count_nonzero(np.asarray(p)) == 1 for _, p, _ in host_std]
+    assert any(greedy) and not all(greedy)  # both temperatures occur
     dev_sp, dev_fin = runs["device"]
     # `play` returns the first 40 finished episodes; the device buffer holds every episode finished so far
-    n_all = sum(len(std) for std, _ in runs[True][0].__dict__.get("_all", [])) if False else None
     dev_std = dev_sp.device_examples.to_examples()
     assert len(dev_std) >= len(host_std)
     for (gb, gp, gv), (wb, wp, wv) in zip(dev_std, host_std):
         assert np.array_equal(gb, np.asarray(wb))
         assert np.array_equal(np.asarray(gp, dtype=np.float64), np.asarray(wp, dtype=np.float64))
-        assert gv == wv
+        assert gv == wv and type(gv) is type(wv)
+    if not use_gnn:
+        return
     dev_gnn = dev_sp.device_gnn_examples.to_examples()
     assert len(dev_gnn) >= len(host_gnn) > 0
     for a, b in zip(dev_gnn, host_gnn):
@@ -134,6 +156,7 @@ def test_device_collection_equals_host_collection():
     # training consumes both device buffers directly
     np.random.seed(0)
     net.train(dev_sp.device_examples, dev_sp.device_gnn_examples)
+
 
 def test_coach_learn_keeps_examples_on_device_and_pickles_the_reference_format(tmp_path):
     from collections import deque

@@ -18,12 +18,12 @@ def make_arena(kind, n, n_games, sims, cpuct, **kw):
 
 
 @pytest.mark.parametrize("tag,G,moves,use_gnn", [("ttt_3", 6, None, False), ("ttt_4", 3, 6, True), ("c4_5", 4, None, True),
-                                                 ("c4_7", 3, 6, False)])
+                                                 ("c4_7", 3, 6, False), ("c4_8", 3, 6, True), ("ttt_5", 3, 6, False)])
 def test_lockstep_games_equal_the_corrected_oracle(tag, G, moves, use_gnn):
     cases.case_lockstep(make_arena, tag, G=G, moves=moves, use_gnn=use_gnn)
 
 
-@pytest.mark.parametrize("tag", ["c4_7", "ttt_4"])
+@pytest.mark.parametrize("tag", ["c4_7", "ttt_4", "c4_8", "ttt_5"])
 def test_compact_leaf_batches_equal_the_corrected_oracle(tag):
     cases.case_compact(make_arena, tag)
 
