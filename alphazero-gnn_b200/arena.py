@@ -42,6 +42,7 @@ class DeviceArena:
         semantics_code(semantics)
         self._open(device)
         self.semantics = semantics
+        self.root_noise = None  # (eta buffer, eps) while attached (set_root_noise)
         self._create_args = dict(kind=kind, n=n, sims_per_move=sims_per_move, cpuct=cpuct, fl_map=fl_map)
         self.kind, self.n, self.G = kind, n, int(n_games)
         self.A = action_size(kind, n)
@@ -92,6 +93,26 @@ class DeviceArena:
         self._check(self.lib.azg_arena_set_semantics(self.handle, code))
         self.semantics = semantics
 
+    def set_root_noise(self, eta, eps):
+        """Attach a [G, A] float64 noise buffer (eta, owned by the caller, kept alive here) or detach it (eta None).
+        From the next launch on, each game's depth-0 PUCT scores use the prior (1 - eps) P + eps eta[g]; the stored P,
+        deeper visits and the exported tables stay clean.  Two-player games only; eps in [0, 1]."""
+        if eta is not None:
+            assert eta.shape == (self.G, self.A) and eta.dtype == torch.float64 and eta.is_contiguous()
+        self._check(self.lib.azg_arena_set_root_noise(self.handle, ptr(eta), float(eps)))
+        self.root_noise = None if eta is None else (eta, float(eps))
+
+    def draw_root_noise(self, seed, ids, alpha, out):
+        """out [G, A] float64 <- Dir(alpha) over the legal moves of every game's current root (zero rows for terminal
+        roots), from Philox4x64-10 keyed by `seed` at the per-game 64-bit `ids` [G] (device int64 / uint64 bit patterns,
+        or a host array): a game's noise depends on (seed, ids[g]) alone."""
+        i = ids if torch.is_tensor(ids) else self.to_device(np.asarray(ids, dtype=np.uint64).view(np.int64), torch.int64)
+        assert i.shape == (self.G,) and i.dtype == torch.int64 and i.is_contiguous()
+        assert out.shape == (self.G, self.A) and out.dtype == torch.float64 and out.is_contiguous()
+        self._check(self.lib.azg_arena_draw_root_noise(self.handle, int(seed) & 0xFFFFFFFFFFFFFFFF, ptr(i), float(alpha),
+                                                      ptr(out), self._stream()))
+        return out
+
     def node_count(self, g=0):
         """entries in game g's table (synchronises)"""
         n = C.c_int(0)
@@ -107,7 +128,7 @@ class DeviceArena:
         nbytes = self.lib.azg_arena_bytes(GAME_KINDS[self.kind], self.n, self.G, capacity, self.max_depth)
         mem = self._alloc(nbytes)
         handle = self._create_handle(mem, nbytes, capacity)
-        self._check(self.lib.azg_arena_copy_from(handle, self.handle, self._stream()))
+        self._check(self.lib.azg_arena_copy_from(handle, self.handle, self._stream()))  # carries semantics and noise
         if self.device.type == "cuda":
             torch.cuda.current_stream().synchronize()  # the copy has read the old buffers before they are released
         self.lib.azg_arena_destroy(self.handle)
@@ -198,7 +219,7 @@ class DeviceArena:
         if st.any():
             bad = np.flatnonzero(st)
             raise RuntimeError(f"arena error in games {bad[:8].tolist()}: code {int(st[bad[0]])} "
-                               f"(4 = node table full, capacity {self.capacity})")
+                               f"(4 = node table full, capacity {self.capacity}; 5 = no root-noise Gamma draw accepted)")
 
     # -- read-back ---------------------------------------------------------------------------------
     def export(self, g):

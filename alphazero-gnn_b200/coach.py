@@ -22,7 +22,7 @@ from random import shuffle
 
 import numpy as np
 
-from .mcts import MCTS, arg, example_symmetries, search_semantics
+from .mcts import MCTS, arg, example_symmetries, game_kind, root_noise, search_semantics
 from .selfplay import BatchedSelfPlay
 
 log = logging.getLogger(__name__)
@@ -98,6 +98,7 @@ class Coach:
         self.game, self.nnet, self.args = game, nnet, args
         self._arena_factory = arena_factory  # tests inject the host check arena
         self.symmetries = example_symmetries(game, search_semantics(args))
+        root_noise(args, game_kind(game))  # b200_root_noise_*: refused here already; BatchedSelfPlay applies them
         self.pnet = None
         self.mcts = self._new_mcts(self.nnet)
         self.trainExamplesHistory = []

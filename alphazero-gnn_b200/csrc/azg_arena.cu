@@ -26,12 +26,15 @@ __device__ __forceinline__ bool group_of(int G, int& g, int& lane, unsigned& mas
   return g < G;
 }
 
+// kNoise: root noise attached (azg_arena_set_root_noise); the launch picks the instance, so searches without noise run
+// kernels that contain no mixing code
+template <int kNoise>
 __global__ void __launch_bounds__(kThreads) arena_select_kernel(AzgArenaView a, AzgState* leaf_states,
                                                                 int32_t* leaf_mask) {
   int g, lane;
   unsigned mask;
   if (!group_of(a.G, g, lane, mask)) return;
-  azg_select_game<kLanes>(a, g, lane, mask, leaf_states, leaf_mask);
+  azg_select_game<kLanes, kNoise>(a, g, lane, mask, leaf_states, leaf_mask);
 }
 
 __global__ void __launch_bounds__(kThreads) arena_expand_backup_kernel(AzgArenaView a, const float* pi,
@@ -40,13 +43,14 @@ __global__ void __launch_bounds__(kThreads) arena_expand_backup_kernel(AzgArenaV
   if (g < a.G) azg_expand_backup_game(a, g, pi, v);
 }
 
+template <int kNoise>
 __global__ void __launch_bounds__(kThreads) arena_select_compact_kernel(AzgArenaView a, AzgState* leaf_states,
                                                                         int32_t* leaf_mask, int32_t* leaf_game,
                                                                         int32_t* leaf_count) {
   int g, lane;
   unsigned mask;
   if (!group_of(a.G, g, lane, mask)) return;
-  azg_select_game<kLanes>(a, g, lane, mask, leaf_states, leaf_mask, leaf_game, leaf_count);
+  azg_select_game<kLanes, kNoise>(a, g, lane, mask, leaf_states, leaf_mask, leaf_game, leaf_count);
 }
 
 __global__ void __launch_bounds__(kThreads) arena_expand_backup_compact_kernel(AzgArenaView a, const float* pi,
@@ -91,6 +95,19 @@ __global__ void arena_get_roots_kernel(AzgArenaView a, AzgState* s) {
 __global__ void arena_begin_kernel(AzgArenaView a, int n_sims) {
   const int g = blockIdx.x * blockDim.x + threadIdx.x;
   if (g < a.G) a.sims_left[g] += n_sims;
+}
+
+__global__ void arena_root_noise_kernel(AzgArenaView a, uint64_t seed, const uint64_t* ids, double alpha, double* eta) {
+  const int g = blockIdx.x * blockDim.x + threadIdx.x;  // one thread per game, actions in ascending order
+  if (g < a.G) azg_root_noise_game(a, g, seed, ids[g], alpha, eta + (size_t)g * a.A);
+}
+
+__global__ void philox_kernel(uint64_t seed, const uint64_t* counters, int64_t n, uint64_t* words) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  uint64_t c[4] = {counters[4 * i], counters[4 * i + 1], counters[4 * i + 2], counters[4 * i + 3]};
+  azg_philox4x64_10(c, seed, 0);
+  for (int j = 0; j < 4; ++j) words[4 * i + j] = c[j];
 }
 
 __global__ void arena_root_stats_kernel(AzgArenaView a, int32_t* N, double* Q, int8_t* qtag) {
@@ -210,12 +227,36 @@ int azg_arena_copy_from(azg_arena* dst, const azg_arena* src, azg_stream stream)
   arena_copy_kernel<<<d.G, 256, 0, (cudaStream_t)stream>>>(d, s);
   AZG_LAUNCH_CHECK();
   dst->view.semantics = s.semantics;  // a grown table continues the search it holds
+  dst->view.noise = s.noise;
+  dst->view.noise_eps = s.noise_eps;
   return AZG_OK;
 }
 
 int azg_arena_set_semantics(azg_arena* a, int semantics) {
   AZG_REQUIRE(a != nullptr, "azg_arena_set_semantics: null arena");
   return azg_view_set_semantics(&a->view, semantics);
+}
+
+int azg_arena_set_root_noise(azg_arena* a, const double* eta, double eps) {
+  AZG_REQUIRE(a != nullptr, "azg_arena_set_root_noise: null arena");
+  return azg_view_set_root_noise(&a->view, eta, eps);
+}
+
+int azg_arena_draw_root_noise(azg_arena* a, uint64_t seed, const uint64_t* ids, double alpha, double* eta, azg_stream stream) {
+  AZG_REQUIRE(a != nullptr, "azg_arena_draw_root_noise: null arena");
+  AZG_REQUIRE(alpha > 0.0 && alpha < INFINITY, "azg_arena_draw_root_noise: alpha must be finite and > 0, got %g", alpha);
+  AZG_REQUIRE(ids && eta, "azg_arena_draw_root_noise: null pointer");
+  arena_root_noise_kernel<<<grid_for(a->view.G, 128), 128, 0, (cudaStream_t)stream>>>(a->view, seed, ids, alpha, eta);
+  AZG_LAUNCH_CHECK();
+  return AZG_OK;
+}
+
+int azg_philox4x64(uint64_t seed, const uint64_t* counters, int64_t n, uint64_t* words, azg_stream stream) {
+  AZG_REQUIRE(n >= 0 && (n == 0 || (counters && words)), "azg_philox4x64: bad argument");
+  if (n == 0) return AZG_OK;
+  philox_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(seed, counters, n, words);
+  AZG_LAUNCH_CHECK();
+  return AZG_OK;
 }
 
 int azg_arena_set_roots(azg_arena* a, const uint64_t* states, azg_stream stream) {
@@ -242,8 +283,8 @@ int azg_arena_begin(azg_arena* a, int n_sims, azg_stream stream) {
 int azg_arena_select(azg_arena* a, uint64_t* leaf_states, int32_t* leaf_mask, azg_stream stream) {
   AZG_REQUIRE(a && leaf_states && leaf_mask, "azg_arena_select: null pointer");
   const int64_t threads = (int64_t)a->view.G * kLanes;
-  arena_select_kernel<<<grid_for(threads, kThreads), kThreads, 0, (cudaStream_t)stream>>>(
-      a->view, (AzgState*)leaf_states, leaf_mask);
+  auto kernel = a->view.noise ? arena_select_kernel<1> : arena_select_kernel<0>;
+  kernel<<<grid_for(threads, kThreads), kThreads, 0, (cudaStream_t)stream>>>(a->view, (AzgState*)leaf_states, leaf_mask);
   AZG_LAUNCH_CHECK();
   return AZG_OK;
 }
@@ -254,8 +295,8 @@ int azg_arena_select_compact(azg_arena* a, uint64_t* leaf_states, int32_t* leaf_
   cudaStream_t st = (cudaStream_t)stream;
   AZG_CUDA_CHECK(cudaMemsetAsync(leaf_count, 0, sizeof(int32_t), st));
   const int64_t threads = (int64_t)a->view.G * kLanes;
-  arena_select_compact_kernel<<<grid_for(threads, kThreads), kThreads, 0, st>>>(a->view, (AzgState*)leaf_states, leaf_mask,
-                                                                                 leaf_game, leaf_count);
+  auto kernel = a->view.noise ? arena_select_compact_kernel<1> : arena_select_compact_kernel<0>;
+  kernel<<<grid_for(threads, kThreads), kThreads, 0, st>>>(a->view, (AzgState*)leaf_states, leaf_mask, leaf_game, leaf_count);
   AZG_LAUNCH_CHECK();
   return AZG_OK;
 }

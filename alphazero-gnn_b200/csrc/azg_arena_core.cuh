@@ -43,6 +43,10 @@ struct AzgArenaView {
   int semantics;  // AZG_SEARCH_REFERENCE / AZG_SEARCH_ALPHAZERO, read by azg_backup only
   int p_f32;  // valid masks are int8 (FrozenLakeGame.py:125): Ps and the PUCT score stay float32 (NEP 50)
   double cpuct;
+  // Dirichlet root noise (azg_arena_set_root_noise): [G, A] float64, caller-owned, NULL = off.  Mixed into the prior
+  // of the depth-0 node only, as (1 - noise_eps) P + noise_eps eta; the stored P is never modified.
+  const double* noise;
+  double noise_eps;
   // per game
   AzgState* root;       // [G]
   int32_t* sims_left;   // [G]
@@ -217,9 +221,11 @@ AZG_HD void azg_backup(const AzgArenaView& a, int g, int depth, AzgVal v) {
   }
 }
 
-// PUCT arg-max over the valid actions of an expanded node, MCTS.py:202-216
+// PUCT arg-max over the valid actions of an expanded node, MCTS.py:202-216.
+// noise_g >= 0 (root of game noise_g, noise on): the prior in both formulas is (1 - eps) P + eps eta[noise_g, act],
+// rounded step by step; the stored P is left as it is.
 template <int W>
-AZG_HD int azg_select_action(const AzgArenaView& a, size_t node, int lane, unsigned mask) {
+AZG_HD int azg_select_action(const AzgArenaView& a, size_t node, int lane, unsigned mask, int noise_g = -1) {
   const uint32_t valids = a.valids[node];
   const double ns = (double)a.ns[node];
   const double sq_visited = azg_dsqrt(ns);                      // math.sqrt(Ns)
@@ -232,7 +238,10 @@ AZG_HD int azg_select_action(const AzgArenaView& a, size_t node, int lane, unsig
       const size_t e = node * a.A + act;
       double u;
       if (!pf32) {  // float64 prior: every factor promotes to float64
-        const double cp = azg_dmul(a.cpuct, a.P[e]);
+        double p = a.P[e];
+        if (noise_g >= 0)
+          p = azg_dadd(azg_dmul(azg_dadd(1.0, -a.noise_eps), p), azg_dmul(a.noise_eps, a.noise[(size_t)noise_g * a.A + act]));
+        const double cp = azg_dmul(a.cpuct, p);
         if (a.qtag[e] != AZG_TAG_NONE)
           u = azg_dadd(a.Q[e], azg_ddiv(azg_dmul(cp, sq_visited), (double)(1 + a.N[e])));
         else
@@ -274,9 +283,12 @@ AZG_HD int azg_select_action(const AzgArenaView& a, size_t node, int lane, unsig
 // simulation budget is spent.
 // leaf_game/leaf_count (optional): compacted output -- games that wait for a prediction claim consecutive
 // slots; leaf_states then holds their positions densely and leaf_game the owning game of each slot.
-template <int W>
+// kNoise: 0 / 1 = root noise off / on, fixed at compile time (the GPU launches pick the kernel, so noise-off kernels carry
+// none of the mixing code); -1 = read a.noise at run time (the host check build).
+template <int W, int kNoise = -1>
 AZG_HD void azg_select_game(const AzgArenaView& a, int g, int lane, unsigned mask, AzgState* leaf_states,
                             int32_t* leaf_mask, int32_t* leaf_game = nullptr, int32_t* leaf_count = nullptr) {
+  const bool noisy = kNoise < 0 ? a.noise != nullptr : kNoise == 1;
   int sims = a.sims_left[g];
   int count = a.node_count[g];
   const bool waiting = a.pending[g] >= 0;
@@ -329,7 +341,7 @@ AZG_HD void azg_select_game(const AzgArenaView& a, int g, int lane, unsigned mas
         need_eval = true;
         break;
       }
-      const int act = azg_select_action<W>(a, node, lane, mask);
+      const int act = azg_select_action<W>(a, node, lane, mask, (noisy && depth == 0) ? g : -1);  // noise: root only
       if (act < 0) break;  // no action: return 0, MCTS.py:218-219
       if (lane == 0) {
         a.path_node[(size_t)g * a.max_depth + depth] = idx;
@@ -439,11 +451,143 @@ static inline int azg_view_set_semantics(AzgArenaView* v, int semantics) {
   v->semantics = semantics;
   return AZG_OK;
 }
+// ---- Dirichlet root noise ----------------------------------------------------------------------------------------
+// Attach (eta != NULL) or detach the [G, A] noise buffer.  eps must lie in [0, 1] (NaN is refused); single-player arenas
+// (FrozenLake: float32 priors, searches that cycle back to the root) take no noise.
+static inline int azg_view_set_root_noise(AzgArenaView* v, const double* eta, double eps) {
+  AZG_REQUIRE(eps >= 0.0 && eps <= 1.0, "azg_arena_set_root_noise: eps must lie in [0, 1], got %g", eps);
+  AZG_REQUIRE(eta == nullptr || (v->two_player && !v->p_f32),
+              "azg_arena_set_root_noise: root noise needs a two-player game (Connect4, TicTacToe)");
+  v->noise = eta;
+  v->noise_eps = eta ? eps : 0.0;
+  return AZG_OK;
+}
+
+// Counter-based generator: Philox4x64-10 (Salmon et al., SC'11), the generator of numpy.random.Philox.  One block of the
+// counter c under the key (k0, k1) gives four 64-bit words.
+AZG_HD uint64_t azg_mulhi64(uint64_t a, uint64_t b) {
+#if defined(__CUDA_ARCH__)
+  return __umul64hi(a, b);
+#else
+  return (uint64_t)(((unsigned __int128)a * b) >> 64);
+#endif
+}
+
+AZG_HD void azg_philox4x64_10(uint64_t c[4], uint64_t k0, uint64_t k1) {
+  for (int r = 0; r < 10; ++r) {
+    if (r > 0) {
+      k0 += 0x9E3779B97F4A7C15ull;
+      k1 += 0xBB67AE8584CAA73Bull;
+    }
+    const uint64_t m0 = 0xD2E7470EE14C6C93ull, m1 = 0xCA5A826395121157ull;
+    const uint64_t hi0 = azg_mulhi64(m0, c[0]), lo0 = m0 * c[0];
+    const uint64_t hi1 = azg_mulhi64(m1, c[2]), lo1 = m1 * c[2];
+    const uint64_t n0 = hi1 ^ c[1] ^ k0, n2 = hi0 ^ c[3] ^ k1;
+    c[0] = n0;
+    c[1] = lo1;
+    c[2] = n2;
+    c[3] = lo0;
+  }
+}
+
+// word -> (0, 1]: ((w >> 11) + 0.5) 2^-53 (the top word of the range rounds to 1.0; 0 is never produced)
+AZG_HD double azg_u01(uint64_t w) { return azg_dmul(azg_dadd((double)(w >> 11), 0.5), 1.1102230246251565e-16); }
+
+#if defined(__CUDA_ARCH__)
+AZG_HD double azg_log(double x) { return log(x); }
+AZG_HD double azg_exp(double x) { return exp(x); }
+AZG_HD double azg_cos(double x) { return cos(x); }
+#else
+static inline double azg_log(double x) { return log(x); }
+static inline double azg_exp(double x) { return exp(x); }
+static inline double azg_cos(double x) { return cos(x); }
+#endif
+
+#define AZG_NOISE_ATTEMPTS 32
+
+// log Gamma(alpha) draw for one (seed, id, action): Marsaglia-Tsang at shape alpha + 1, boosted back to alpha in log
+// space (log u4 / alpha), so small alpha neither underflows nor divides 0 by 0.  Attempt k reads the block at counter
+// (id, action, k, 0).  Returns the accepted attempt, or -1 when none of the AZG_NOISE_ATTEMPTS was accepted.
+AZG_HD int azg_log_gamma(uint64_t seed, uint64_t id, int action, double alpha, double* lg) {
+  const double d = azg_dadd(azg_dadd(alpha, 1.0), -(1.0 / 3.0));
+  const double c = azg_ddiv(1.0, azg_dsqrt(azg_dmul(9.0, d)));
+  for (int k = 0; k < AZG_NOISE_ATTEMPTS; ++k) {
+    uint64_t w[4] = {id, (uint64_t)action, (uint64_t)k, 0};
+    azg_philox4x64_10(w, seed, 0);
+    const double u1 = azg_u01(w[0]), u2 = azg_u01(w[1]), u3 = azg_u01(w[2]), u4 = azg_u01(w[3]);
+    const double x = azg_dmul(azg_dsqrt(azg_dmul(-2.0, azg_log(u1))), azg_cos(azg_dmul(u2, 6.283185307179586)));
+    const double t = azg_dadd(1.0, azg_dmul(c, x));
+    const double v = azg_dmul(azg_dmul(t, t), t);
+    if (!(v > 0.0)) continue;
+    const double lv = azg_log(v);
+    const double rhs = azg_dadd(azg_dadd(azg_dadd(azg_dmul(azg_dmul(x, x), 0.5), d), -azg_dmul(d, v)), azg_dmul(d, lv));
+    if (azg_log(u3) < rhs) {
+      *lg = azg_dadd(azg_dadd(azg_log(d), lv), azg_ddiv(azg_log(u4), alpha));
+      return k;
+    }
+  }
+  return -1;
+}
+
+// eta ~ Dir(alpha) over the legal moves of game g's root, written to eta_row [A] (also the scratch of the log-Gammas):
+// eta_a = exp(lg_a - max) / sum_b exp(lg_b - max), summed in ascending action order; 0 on illegal actions, a zero row
+// for a terminal root.  Running out of attempts sets the sticky status AZG_ERR_NOISE and leaves a zero row.
+AZG_HD void azg_root_noise_game(const AzgArenaView& a, int g, uint64_t seed, uint64_t id, double alpha, double* eta_row) {
+  const AzgState s = a.root[g];
+  const uint32_t valids = azg_ended(a.rules, s).tag == AZG_TAG_NONE ? azg_valids(a.rules, s) : 0u;
+  double mx = -INFINITY;
+  bool ok = true;
+  for (int i = 0; i < a.A; ++i) {
+    double lg = 0.0;
+    if ((valids >> i) & 1u) {
+      if (azg_log_gamma(seed, id, i, alpha, &lg) < 0) {
+        ok = false;
+        break;
+      }
+      if (lg > mx) mx = lg;
+    }
+    eta_row[i] = lg;
+  }
+  if (!ok) {
+    a.status[g] = AZG_ERR_NOISE;
+    for (int i = 0; i < a.A; ++i) eta_row[i] = 0.0;
+    return;
+  }
+  double sum = 0.0;
+  for (int i = 0; i < a.A; ++i) {
+    const double e = ((valids >> i) & 1u) ? azg_exp(azg_dadd(eta_row[i], -mx)) : 0.0;
+    eta_row[i] = e;
+    sum = azg_dadd(sum, e);
+  }
+  for (int i = 0; i < a.A; ++i) eta_row[i] = ((valids >> i) & 1u) ? azg_ddiv(eta_row[i], sum) : 0.0;
+}
+
 #if !defined(__CUDACC__)
 // The host check build (tests/hostcheck) compiles this file with a host compiler and binds every azg_arena_* entry
 // point of include/azgnn_b200.h under an `azgh_` name.  Its handle is a struct whose first and only member is the
 // view, so the handle points at the view.
 extern "C" int azgh_arena_set_semantics(AzgArenaView* a, int semantics) { return azg_view_set_semantics(a, semantics); }
+extern "C" int azgh_arena_set_root_noise(AzgArenaView* a, const double* eta, double eps) {
+  AZG_REQUIRE(a != nullptr, "azg_arena_set_root_noise: null arena");
+  return azg_view_set_root_noise(a, eta, eps);
+}
+// the same sampler on the host (host libm: log / cos / exp may differ from the device's in the last bit)
+extern "C" int azgh_arena_draw_root_noise(AzgArenaView* a, uint64_t seed, const uint64_t* ids, double alpha, double* eta,
+                                          void*) {
+  AZG_REQUIRE(a != nullptr, "azg_arena_draw_root_noise: null arena");
+  AZG_REQUIRE(alpha > 0.0 && alpha < INFINITY, "azg_arena_draw_root_noise: alpha must be finite and > 0, got %g", alpha);
+  AZG_REQUIRE(ids && eta, "azg_arena_draw_root_noise: null pointer");
+  for (int g = 0; g < a->G; ++g) azg_root_noise_game(*a, g, seed, ids[g], alpha, eta + (size_t)g * a->A);
+  return AZG_OK;
+}
+extern "C" int azgh_philox4x64(uint64_t seed, const uint64_t* counters, int64_t n, uint64_t* words, void*) {
+  for (int64_t i = 0; i < n; ++i) {
+    uint64_t c[4] = {counters[4 * i], counters[4 * i + 1], counters[4 * i + 2], counters[4 * i + 3]};
+    azg_philox4x64_10(c, seed, 0);
+    for (int j = 0; j < 4; ++j) words[4 * i + j] = c[j];
+  }
+  return AZG_OK;
+}
 #endif
 
 // ---- table growth: copy game g from `s` into the larger `d` (same game, A, max_depth; d.cap >= s.cap) ------------

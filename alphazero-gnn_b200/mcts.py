@@ -38,6 +38,33 @@ def search_semantics(args):
     return sem
 
 
+def root_noise(args, kind):
+    """args.b200_root_noise_eps / b200_root_noise_alpha -> (alpha, eps) of the self-play root noise, or None when it is
+    off (eps absent or 0).  eps: a number in [0, 1]; alpha: a finite number > 0, required when eps > 0.  Two-player
+    games only (FrozenLake refuses eps > 0).  Anything else raises ValueError."""
+    import math
+
+    def number(name, value):
+        if isinstance(value, bool) or not isinstance(value, (int, float, np.integer, np.floating)) or math.isnan(value):
+            raise ValueError(f"{name} must be a number, got {value!r}")
+        return float(value)
+    eps, alpha = arg(args, "b200_root_noise_eps"), arg(args, "b200_root_noise_alpha")
+    eps = 0.0 if eps is None else number("b200_root_noise_eps", eps)
+    if not 0.0 <= eps <= 1.0:
+        raise ValueError(f"b200_root_noise_eps must lie in [0, 1], got {eps!r}")
+    if alpha is not None:
+        alpha = number("b200_root_noise_alpha", alpha)
+        if not (alpha > 0 and math.isfinite(alpha)):
+            raise ValueError(f"b200_root_noise_alpha must be finite and > 0, got {alpha!r}")
+    if eps == 0.0:
+        return None
+    if alpha is None:
+        raise ValueError("b200_root_noise_eps > 0 needs b200_root_noise_alpha")
+    if kind == "frozenlake":
+        raise ValueError("root noise is for two-player games; FrozenLake takes no b200_root_noise_eps")
+    return alpha, eps
+
+
 def example_symmetries(game, semantics):
     """The symmetric forms self-play turns each position into: the game's own `getSymmetries`, except for Connect4 in
     the "alphazero" semantics, whose mirror reverses the columns (games.Connect4Game(mirror_columns=True))."""
@@ -169,7 +196,7 @@ class BatchedMCTS:
         self.gnn_predictions = [dict() for _ in range(n_games)]
         self.leaf_evals = 0          # positions submitted for evaluation (host path: exact; device paths: see below)
         self._leaf_total = None      # compact path: exact count accumulated on the device (int64 [1], updated in place)
-        self._graphs = {}            # n_sims -> "warm" | (CUDAGraph, weights version): captured searches (search(graph=True))
+        self._graphs = {}            # n_sims (noise on: + buffer, eps) -> "warm" | (CUDAGraph, weights version): captured searches (search(graph=True))
 
     # ------------------------------------------------------------------ roots
     def reset(self, game_ids=None):
@@ -223,11 +250,14 @@ class BatchedMCTS:
         (loads kernels, packs weights, settles the precision guard); second call: captured, then replayed; a graph is
         dropped when the network's weights change (it holds the address of the packed weight images)."""
         version = getattr(self.nnet, "weights_version", 0)
-        st = self._graphs.get(n_sims)
+        # a captured launch holds the arena view by value, root-noise buffer and eps included
+        noise = getattr(self.arena, "root_noise", None)
+        key = n_sims if noise is None else (n_sims, noise[0].data_ptr(), noise[1])
+        st = self._graphs.get(key)
         if isinstance(st, tuple) and st[1] != version:
             st = None
         if st is None:
-            self._graphs[n_sims] = "warm"
+            self._graphs[key] = "warm"
             return False
         if st == "warm":
             if self._leaf_total is None:
@@ -236,7 +266,7 @@ class BatchedMCTS:
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
                 self._search_rounds(n_sims)
-            st = self._graphs[n_sims] = (g, version)
+            st = self._graphs[key] = (g, version)
         st[0].replay()
         return True
 

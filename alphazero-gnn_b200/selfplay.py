@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 from ._lib import ptr
-from .mcts import BatchedMCTS, arg, example_symmetries, pack_states
+from .mcts import BatchedMCTS, arg, example_symmetries, pack_states, root_noise
 
 EPS = 1e-8
 
@@ -92,6 +92,16 @@ class BatchedSelfPlay:
         self.kind, self.n, self.A = self.mcts.kind, self.mcts.n, self.mcts.A
         self.symmetries = example_symmetries(game, self.mcts.semantics)
         self.rng = np.random.default_rng(seed)
+        # Dirichlet root noise (b200_root_noise_alpha / b200_root_noise_eps, off by default): one [G, A] buffer attached to
+        # the arena once and redrawn on the device before every move's numMCTSSims searches; the move's expand_by
+        # searches continue the same tree from the same root with the same noise.  The draw of a move depends on
+        # (seed, episode index, episode step) alone, never on the slot the episode plays in.
+        self.seed = int(seed)
+        self.noise = root_noise(args, self.kind)
+        if self.noise is not None:
+            ar = self.mcts.arena
+            self.eta = torch.zeros(self.G, self.A, dtype=torch.float64, device=ar.device)
+            ar.set_root_noise(self.eta, self.noise[1])
         # collect_examples: False (throughput runs), True (host lists, the reference's tuples), or "device": standard
         # examples are assembled on the GPU (replay.DeviceExamples: history in HBM, symmetries + value signing in one
         # kernel per batch of finished episodes) and `play` returns them as ONE DeviceExamples
@@ -146,6 +156,14 @@ class BatchedSelfPlay:
                                   torch.zeros(tc, G_, A_, dtype=torch.float64, device=dev), torch.zeros(tc, G_, dtype=torch.float64, device=dev),
                                   torch.zeros(tc, G_, dtype=torch.int8, device=dev))
         self._start_all()
+
+    def _search_move(self, n_sims, steps, check=True):
+        """numMCTSSims searches of the move at episode step `steps` [G] of every game, with fresh root noise when it is on:
+        per game id (episode index << 32) | episode step"""
+        if self.noise is not None:
+            ids = (self.ep_index.astype(np.uint64) << np.uint64(32)) | np.asarray(steps).astype(np.uint64)
+            self.mcts.arena.draw_root_noise(self.seed, ids, self.noise[0], self.eta)
+        self.mcts.search(n_sims, check=check)
 
     # ------------------------------------------------------------------ episode bookkeeping
     def _start_all(self):
@@ -238,7 +256,7 @@ class BatchedSelfPlay:
             m.arena.check_status()  # the searches queued at the end of the previous move
             self._inflight = False
         else:
-            m.search(n_sims)
+            self._search_move(n_sims, self.step)
         N, _, _ = m.root_stats()
         recs, pending, launched = None, None, False
         if self.use_gnn and m.device_eval:
@@ -301,7 +319,7 @@ class BatchedSelfPlay:
             self.episodes_done += len(done)
             self._restart(done)
         if m.device_eval:  # next move's searches: the GPU works while the host finishes this move's records
-            m.search(n_sims, check=False)
+            self._search_move(n_sims, self.step + 1, check=False)
             self._inflight = True
         if self.device_collect:
             if readback is not None:
@@ -327,7 +345,7 @@ class BatchedSelfPlay:
         if self._inflight:
             self._inflight = False  # the searches queued at the end of the previous move; status is read below
         else:
-            m.search(n_sims, check=False)
+            self._search_move(n_sims, self.step, check=False)
         n0 = ar.root_stats()[0].clone()
         n1 = q1 = t1 = v0 = None
         if self.use_gnn:  # expand_tree (MCTS.py:60-149): standard root value, expand_by more searches
@@ -399,7 +417,7 @@ class BatchedSelfPlay:
                 self.player[d] = 1
                 self.ep_index[d] = self._next_ep + np.arange(len(again))
                 self._next_ep += len(again)
-        m.search(n_sims, check=False)  # next move's searches run while the host emits the finished episodes
+        self._search_move(n_sims, self.step + 1, check=False)  # next move's searches run while the host emits the finished episodes
         self._inflight = True
         if keep:
             self._finish_device(keep, ended, lens, cur)

@@ -34,6 +34,7 @@ extern "C" {
 #define AZG_ERR_CUDA 2      /* CUDA runtime error (message in azg_last_error) */
 #define AZG_ERR_DEVICE 3    /* not an sm_100 device / no device */
 #define AZG_ERR_CAPACITY 4  /* arena node table full */
+#define AZG_ERR_NOISE 5     /* root noise: no Gamma draw accepted in 32 attempts (probability below 1e-40) */
 
 #define AZG_GAME_CONNECT4 0
 #define AZG_GAME_TICTACTOE 1
@@ -326,7 +327,7 @@ int azg_arena_destroy(azg_arena* a);
  * arenaCompare games (Coach.py:128-142), so a table can outgrow any fixed capacity.  Copies every game of `src` (nodes,
  * edges, per-game search state) into `dst`, an arena of the same game / n_games / max_depth created with a larger
  * capacity_nodes, and rebuilds the hash for the new size; node indices are preserved.  `dst` takes `src`'s search
- * semantics. */
+ * semantics and root noise attachment. */
 int azg_arena_copy_from(azg_arena* dst, const azg_arena* src, azg_stream stream);
 /* Backup semantics of a two-player search (single-player games are unaffected).  AZG_SEARCH_REFERENCE (the default
  * of a new arena): Qsa(s,a) holds the child's value before it is negated (MCTS.py:228-240), i.e. from the point of
@@ -336,6 +337,21 @@ int azg_arena_copy_from(azg_arena* dst, const azg_arena* src, azg_stream stream)
 #define AZG_SEARCH_REFERENCE 0
 #define AZG_SEARCH_ALPHAZERO 1
 int azg_arena_set_semantics(azg_arena* a, int semantics);
+/* Dirichlet noise at the root (two-player games only; opt-in, off in a new arena).  Attaches the caller-owned device
+ * buffer eta [n_games, A] float64 (NULL detaches): from the next launch on, the PUCT scores of each game's depth-0 node
+ * use the prior (1 - eps) P(root, a) + eps eta[g, a], with every rounding spelled out.  The stored P is never modified,
+ * so deeper visits, azg_arena_export and expand_tree read the clean prior.  Refused (AZG_ERR_INVALID): eps outside
+ * [0, 1] or NaN, a buffer on a single-player arena.  `azg_arena_copy_from` carries the attachment into a grown table. */
+int azg_arena_set_root_noise(azg_arena* a, const double* eta, double eps);
+/* eta [n_games, A] ~ Dir(alpha) over the legal moves of each game's current root, one thread per game:
+ * log Gamma(alpha) per legal action by Marsaglia-Tsang at shape alpha + 1 with the boost in log space, at most 32
+ * attempts (running out sets the sticky status AZG_ERR_NOISE); uniforms from Philox4x64-10 under the key (seed, 0) at
+ * counter (ids[g], action, attempt, 0), so a game's draw depends on (seed, ids[g]) alone, never on its slot.
+ * eta_a = exp(lg_a - max) / sum_b exp(lg_b - max) in ascending action order; 0 on illegal actions; a terminal root gets
+ * a zero row.  ids: device uint64 [n_games].  Refuses alpha <= 0 or non-finite. */
+int azg_arena_draw_root_noise(azg_arena* a, uint64_t seed, const uint64_t* ids, double alpha, double* eta, azg_stream stream);
+/* the generator above, exposed for parity tests against numpy.random.Philox: counters [n,4] -> words [n,4] */
+int azg_philox4x64(uint64_t seed, const uint64_t* counters, int64_t n, uint64_t* words, azg_stream stream);
 int azg_arena_action_size(const azg_arena* a);
 /* new MCTS object for the listed games (Coach.py:96): clear their tables.  game_ids: device
  * int32 [count], or NULL = all games. */
