@@ -119,6 +119,7 @@ SIGNATURES = {
     "azg_arena_set_root_noise": (_i, [_vp, _vp, _d]),
     "azg_arena_draw_root_noise": (_i, [_vp, C.c_uint64, _vp, _d, _vp, _vp]),
     "azg_philox4x64": (_i, [C.c_uint64, _vp, _i64, _vp, _vp]),
+    "azg_rollout_eval": (_i, [_i, _i, _vp, _vp, _i64, _vp, _i, C.c_uint64, _vp, _vp, _vp]),
     "azg_arena_action_size": (_i, [_vp]),
     "azg_arena_reset": (_i, [_vp, _vp, _i, _vp]),
     "azg_arena_set_roots": (_i, [_vp, _vp, _vp]),

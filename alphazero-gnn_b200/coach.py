@@ -23,9 +23,12 @@ from random import shuffle
 import numpy as np
 
 from .mcts import MCTS, arg, example_symmetries, game_kind, root_noise, search_semantics
+from .rollout import eval_settings
 from .selfplay import BatchedSelfPlay
 
 log = logging.getLogger(__name__)
+
+ROLLOUT_EVAL_SEED = 0x5EED  # the rollout opponent of `b200_eval_rollout_*` (rank r: this + r): the same at every iteration
 
 
 class _CheckpointWriter:
@@ -99,6 +102,12 @@ class Coach:
         self._arena_factory = arena_factory  # tests inject the host check arena
         self.symmetries = example_symmetries(game, search_semantics(args))
         root_noise(args, game_kind(game))  # b200_root_noise_*: refused here already; BatchedSelfPlay applies them
+        self.rollout_eval = eval_settings(args, game_kind(game))  # (games, sims, playouts) or None
+        if self.rollout_eval is not None and arena_factory is not None:
+            raise ValueError("b200_eval_rollout_games needs the CUDA arena (the rollout player runs on the GPU only)")
+        self._rollout = None
+        self.rollout_result = None   # (wins, draws, losses) of the network in the last evaluation
+        self.rollout_history = []    # (iteration, wins, draws, losses) per iteration
         self.pnet = None
         self.mcts = self._new_mcts(self.nnet)
         self.trainExamplesHistory = []
@@ -168,6 +177,34 @@ class Coach:
             else:
                 nw += 1
         return pw, nw, dr
+
+    def rollout_match(self):
+        """The network (searching with the Coach's settings) against the fixed rollout player (`b200_eval_rollout_sims`
+        simulations, `b200_eval_rollout_playouts` playouts per leaf, always the corrected "alphazero" backup: the
+        reference's makes every node prefer its opponent's best move, SURVEY section 0 item 1), in
+        `b200_eval_rollout_games` games with first moves alternating, sharded over the ranks like the arena.  Returns the
+        network's (wins, draws, losses) over all ranks.  The global NumPy RNG that the arena's tie-breaks draw from is
+        restored afterwards, so the evaluation leaves the training run as it was."""
+        import torch
+        from .pit import BatchedArena, with_args
+        from .rollout import RolloutPlayer
+        n_games, sims, playouts = self.rollout_eval
+        rank, world = self._world()
+        if self._rollout is None:
+            self._rollout = RolloutPlayer(self.game, playouts, seed=ROLLOUT_EVAL_SEED + rank)  # ranks play distinct games
+        r_args = with_args(self.args, numMCTSSims=sims, use_gnn=False, b200_search_semantics="alphazero")
+        mine = 2 * ((n_games // 2 + world - 1 - rank) // world) if world > 1 else n_games
+        state = np.random.get_state()
+        try:
+            wins, losses, draws = BatchedArena(self.game, self.nnet, self._rollout, self.args, args2=r_args).playGames(mine)
+        finally:
+            np.random.set_state(state)
+        if world > 1:
+            import torch.distributed as dist
+            c = torch.tensor([wins, draws, losses], dtype=torch.int64, device=self.nnet.device)
+            dist.all_reduce(c)
+            wins, draws, losses = (int(x) for x in c.tolist())
+        return wins, draws, losses
 
     def getCheckpointFile(self, iteration):
         return f"checkpoint_{iteration}" + ("_gnn" if self._use_gnn() else "") + ".pth.tar"
@@ -374,5 +411,11 @@ class Coach:
                 else:
                     self.nnet.save_checkpoint(folder=folder, filename=self.getCheckpointFile(i))
                     self.nnet.save_checkpoint(folder=folder, filename=best)
+            if self.rollout_eval is not None:  # the network kept by the decision above against the fixed yardstick
+                t6 = sync()
+                self.rollout_result = self.rollout_match()
+                self.rollout_history.append((i,) + self.rollout_result)
+                self.timings["rollout_eval_s"] = sync() - t6
+                log.info("VS ROLLOUT-MCTS (%d sims, %d playouts) W/D/L : %d / %d / %d" % (self.rollout_eval[1:] + self.rollout_result))
         if writer is not None:
             writer.flush()

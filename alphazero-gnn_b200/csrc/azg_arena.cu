@@ -144,6 +144,41 @@ __global__ void rules_eval_kernel(AzgRules r, const AzgState* states, int64_t B,
   }
 }
 
+// Rollout leaf values: `tpr` threads per leaf (the power of two >= playouts, at most kRolloutThreads), one playout per
+// thread and round, kRolloutThreads / tpr leaves per CTA.  Outcomes are summed as integers (warp shuffles, then one
+// shared-memory atomic per warp and leaf), so v does not depend on the order of the reduction.
+constexpr int kRolloutThreads = 256;
+
+__global__ void __launch_bounds__(kRolloutThreads) rollout_eval_kernel(AzgRules r, const AzgState* states,
+                                                                       const int32_t* games, int64_t rows,
+                                                                       const int32_t* count, int playouts, int tpr,
+                                                                       uint64_t seed, float* pi, float* v) {
+  const int rpb = kRolloutThreads / tpr;
+  const int64_t first = (int64_t)blockIdx.x * rpb;
+  const int64_t live = count ? min((int64_t)*count, rows) : rows;
+  if (first >= live) return;  // the whole CTA is past the leaf count
+  __shared__ int sums[kRolloutThreads];
+  const int slot = threadIdx.x / tpr, lane = threadIdx.x % tpr;
+  const int64_t row = first + slot;
+  const bool on = row < live;
+  if (lane == 0) sums[slot] = 0;
+  __syncthreads();
+  AzgState s;
+  s.mine = s.theirs = 0;
+  int acc = 0;
+  if (on) {
+    s = states[row];
+    const uint32_t g = games ? (uint32_t)games[row] : (uint32_t)row;
+    for (int p = lane; p < playouts; p += tpr) acc += azg_rollout_outcome(r, s, seed, g, (uint32_t)p);
+  }
+  for (int off = min(tpr, 32) / 2; off > 0; off >>= 1) acc += __shfl_xor_sync(0xFFFFFFFFu, acc, off);
+  if (on && (lane & 31) == 0) atomicAdd(&sums[slot], acc);
+  __syncthreads();
+  if (!on) return;
+  if (lane == 0) v[row] = __fdiv_rn((float)sums[slot], (float)playouts);
+  azg_rollout_policy(r, s, pi + row * r.A, lane, tpr);
+}
+
 inline int grid_for(int64_t n, int threads) { return (int)((n + threads - 1) / threads); }
 
 }  // namespace
@@ -255,6 +290,22 @@ int azg_philox4x64(uint64_t seed, const uint64_t* counters, int64_t n, uint64_t*
   AZG_REQUIRE(n >= 0 && (n == 0 || (counters && words)), "azg_philox4x64: bad argument");
   if (n == 0) return AZG_OK;
   philox_kernel<<<grid_for(n, 256), 256, 0, (cudaStream_t)stream>>>(seed, counters, n, words);
+  AZG_LAUNCH_CHECK();
+  return AZG_OK;
+}
+
+int azg_rollout_eval(int game, int n, const uint64_t* states, const int32_t* games, int64_t rows, const int32_t* count,
+                     int playouts, uint64_t seed, float* pi, float* v, azg_stream stream) {
+  AzgRules r;
+  const int rc = azg_rollout_setup(&r, game, n, playouts);
+  if (rc != AZG_OK) return rc;
+  AZG_REQUIRE(rows >= 0 && rows <= 0x7FFFFFFF, "azg_rollout_eval: rows must lie in [0, 2^31), got %lld", (long long)rows);
+  AZG_REQUIRE(rows == 0 || (states && pi && v), "azg_rollout_eval: null pointer");
+  if (rows == 0) return AZG_OK;
+  int tpr = 1;
+  while (tpr < playouts && tpr < kRolloutThreads) tpr <<= 1;
+  rollout_eval_kernel<<<grid_for(rows, kRolloutThreads / tpr), kRolloutThreads, 0, (cudaStream_t)stream>>>(
+      r, (const AzgState*)states, games, rows, count, playouts, tpr, seed, pi, v);
   AZG_LAUNCH_CHECK();
   return AZG_OK;
 }

@@ -590,6 +590,102 @@ extern "C" int azgh_philox4x64(uint64_t seed, const uint64_t* counters, int64_t 
 }
 #endif
 
+// ---- rollout baseline: leaves valued by uniformly random playouts ------------------------------------------------
+#define AZG_ROLLOUT_MAX_PLAYOUTS 4096
+
+// Arguments of azg_rollout_eval, checked once for the library and the host check build; fills *r on success.
+static inline int azg_rollout_setup(AzgRules* r, int game, int n, int playouts) {
+  AZG_REQUIRE(game == AZG_GAME_CONNECT4 || game == AZG_GAME_TICTACTOE,
+              "azg_rollout_eval: two-player games only (Connect4, TicTacToe), got game %d", game);
+  AZG_REQUIRE(game == AZG_GAME_CONNECT4 ? (n >= 4 && n <= 8) : (n >= 3 && n <= 5),
+              "azg_rollout_eval: unsupported board size %d (Connect4 4..8, TicTacToe 3..5)", n);
+  AZG_REQUIRE(playouts >= 1 && playouts <= AZG_ROLLOUT_MAX_PLAYOUTS, "azg_rollout_eval: playouts must lie in [1, %d], got %d",
+              AZG_ROLLOUT_MAX_PLAYOUTS, playouts);
+  AZG_REQUIRE(azg_rules_init(r, game, n, nullptr) == 0, "azg_rollout_eval: unsupported game %d / size %d", game, n);
+  return AZG_OK;
+}
+
+// One uniformly random playout from s: +1 / 0 / -1 for the player to move at s (draws, Connect4's 1e-4 included, are 0).
+// Ply t reads word t % 4 of the Philox4x64-10 block at counter (s.mine, s.theirs, (game << 32) | playout, t / 4) under the
+// key (seed, 1) -- root noise uses (seed, 0), so the streams share no block -- and plays the j-th legal action in
+// ascending order, j = mulhi64(word, k) for k legal actions.  The game is checked with azg_ended at ply 0 only: a
+// position that has not ended can only end by the mover's new stone, so later plies test the lines through it (TicTacToe)
+// or the mover's stones (Connect4), and a full board.  That is azg_ended's answer by construction (the host spec test pins
+// it); the outcome of the state reached after ply t is negated t + 1 times, because the canonical board flips every ply.
+AZG_HD int azg_rollout_outcome(const AzgRules& r, AzgState s, uint64_t seed, uint32_t game, uint32_t playout) {
+  const AzgVal e0 = azg_ended(r, s);
+  if (e0.tag != AZG_TAG_NONE) return e0.d == 1.0 ? 1 : (e0.d == -1.0 ? -1 : 0);
+  const bool c4 = r.game == AZG_GAME_CONNECT4;
+  const int n = r.n;
+  uint64_t full = r.board_mask;  // Connect4: no legal column once every top cell is taken
+  if (c4) {
+    full = 0;
+    for (int x = 0; x < n; ++x) full |= 1ull << (x * n + n - 1);
+  }
+  const uint64_t c0 = s.mine, c1 = s.theirs, c2 = ((uint64_t)game << 32) | playout;
+  uint64_t w[4] = {0, 0, 0, 0};
+  for (int t = 0;; ++t) {
+    if ((t & 3) == 0) {
+      w[0] = c0;
+      w[1] = c1;
+      w[2] = c2;
+      w[3] = (uint64_t)(t >> 2);
+      azg_philox4x64_10(w, seed, 1);
+    }
+    const int q = t & 3;  // selects by value: an indexed w[] would live in local memory
+    const uint64_t word = q == 0 ? w[0] : q == 1 ? w[1] : q == 2 ? w[2] : w[3];
+    uint32_t m = azg_valids(r, s);
+    int j = (int)azg_mulhi64(word, (uint64_t)azg_popc64(m));
+    while (j-- > 0) m &= m - 1;
+    const int a = azg_popc64((uint64_t)((m & (0u - m)) - 1u));  // index of the lowest remaining set bit
+    const AzgState nx = azg_next(r, s, a);
+    const uint64_t mover = nx.theirs;
+    bool won;
+    if (c4) {
+      won = azg_c4_wins(r, mover);
+    } else {  // lines through cell a = x * n + y: row y, column x, and the diagonals it lies on
+      const int x = a / n, y = a % n;
+      won = (mover & r.lines[y]) == r.lines[y] || (mover & r.lines[n + x]) == r.lines[n + x] ||
+            (x == y && (mover & r.lines[2 * n]) == r.lines[2 * n]) ||
+            (x + y == n - 1 && (mover & r.lines[2 * n + 1]) == r.lines[2 * n + 1]);
+    }
+    if (won) return (t & 1) ? -1 : 1;  // the mover of ply t is the player to move at s when t is even
+    if (((nx.mine | nx.theirs) & full) == full) return 0;
+    s = nx;
+  }
+}
+
+// pi row for a leaf: 1/k (float32, rounded to nearest) on its k legal moves (azg_valids), 0 elsewhere
+AZG_HD void azg_rollout_policy(const AzgRules& r, AzgState s, float* pi_row, int lane, int lanes) {
+  const uint32_t m = azg_valids(r, s);
+  const float p = azg_fdiv(1.0f, (float)azg_popc64(m));
+  for (int a = lane; a < r.A; a += lanes) pi_row[a] = ((m >> a) & 1u) ? p : 0.0f;
+}
+
+#if !defined(__CUDACC__)
+// host check build of azg_rollout_eval (host pointers, rows one after the other)
+extern "C" int azgh_rollout_eval(int game, int n, const uint64_t* states, const int32_t* games, int64_t rows,
+                                 const int32_t* count, int playouts, uint64_t seed, float* pi, float* v, void*) {
+  AzgRules r;
+  const int rc = azg_rollout_setup(&r, game, n, playouts);
+  if (rc != AZG_OK) return rc;
+  AZG_REQUIRE(rows >= 0 && rows <= 0x7FFFFFFF, "azg_rollout_eval: rows must lie in [0, 2^31), got %lld", (long long)rows);
+  AZG_REQUIRE(rows == 0 || (states && pi && v), "azg_rollout_eval: null pointer");
+  const int64_t live = count ? (*count < rows ? *count : rows) : rows;
+  for (int64_t i = 0; i < live; ++i) {
+    AzgState s;
+    s.mine = states[2 * i];
+    s.theirs = states[2 * i + 1];
+    const uint32_t g = games ? (uint32_t)games[i] : (uint32_t)i;
+    int sum = 0;
+    for (int p = 0; p < playouts; ++p) sum += azg_rollout_outcome(r, s, seed, g, (uint32_t)p);
+    v[i] = azg_fdiv((float)sum, (float)playouts);
+    azg_rollout_policy(r, s, pi + i * r.A, 0, 1);
+  }
+  return AZG_OK;
+}
+#endif
+
 // ---- table growth: copy game g from `s` into the larger `d` (same game, A, max_depth; d.cap >= s.cap) ------------
 // part 1 (any number of lanes): clear d's hash slots and copy the node and edge arrays verbatim (node indices are kept)
 AZG_HD void azg_copy_game_nodes(const AzgArenaView& d, const AzgArenaView& s, int g, int lane, int lanes) {

@@ -210,12 +210,16 @@ class BatchedMCTS:
         return [unpack_state(self.kind, self.n, r) for r in roots]
 
     # ------------------------------------------------------------------ leaf evaluation
-    def _evaluate_device(self, leaf_states, count=None):
+    def _evaluate_device(self, leaf_states, count=None, games=None):
+        """games: the compact leaf_game buffer, handed only to evaluators that declare `keyed_by_game` (their outputs
+        depend on the game a leaf belongs to, rollout.RolloutPlayer); networks get the same calls as without it"""
         # use_gnn: MCTS.py:169-176 calls predict AND predict_with_gnn at every leaf but searches with the GNN prediction
         # only; the standard prediction is read back for ROOTS alone (expand_tree, MCTS.py:108-111), and those are
         # evaluated by _root_std_values.  The device path therefore skips the unused standard heads at the leaves.
         mask = _lib.EVAL_GNN if self.use_gnn else _lib.EVAL_STD
         kw = self._search_kw()
+        if games is not None and getattr(self.nnet, "keyed_by_game", False):
+            kw["games"] = games
         out = self.nnet.forward_states(leaf_states, mask, count=count, **kw) if count is not None else \
             self.nnet.forward_states(leaf_states, mask, **kw)
         return (out["pi_gnn"], out["v_gnn"]) if self.use_gnn else (out["pi"], out["v"])
@@ -274,8 +278,8 @@ class BatchedMCTS:
         ar = self.arena
         ar.begin(n_sims)
         for _ in range(n_sims):  # every round retires >= 1 simulation per game that has budget
-            leaf_states, _game, count = ar.select_compact()
-            pi, v = self._evaluate_device(leaf_states, count)
+            leaf_states, leaf_game, count = ar.select_compact()
+            pi, v = self._evaluate_device(leaf_states, count, leaf_game)
             ar.expand_backup_compact(pi, v)
             if self._leaf_total is None:
                 self._leaf_total = torch.zeros(1, dtype=torch.int64, device=ar.device)

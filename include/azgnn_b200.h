@@ -352,6 +352,17 @@ int azg_arena_set_root_noise(azg_arena* a, const double* eta, double eps);
 int azg_arena_draw_root_noise(azg_arena* a, uint64_t seed, const uint64_t* ids, double alpha, double* eta, azg_stream stream);
 /* the generator above, exposed for parity tests against numpy.random.Philox: counters [n,4] -> words [n,4] */
 int azg_philox4x64(uint64_t seed, const uint64_t* counters, int64_t n, uint64_t* words, azg_stream stream);
+/* Rollout baseline: the leaf evaluation of an MCTS player that needs no network.  For every row i below the leaf count,
+ * v[i] = (sum of `playouts` outcomes) / playouts (float32, one rounding; the sum is an exact integer) and pi [rows, A] =
+ * 1/k (float32) on the k legal moves (getValidMoves) of states[i], 0 elsewhere.  An outcome is +1 / 0 / -1 for the player
+ * to move at states[i] after uniformly random play to the end (a draw, Connect4's 1e-4 included, is 0; a terminal state
+ * is its own outcome); ply t of playout p reads word t % 4 of the Philox4x64-10 block at counter
+ * (mine, theirs, (games[i] << 32) | p, t / 4) under the key (seed, 1) and plays the j-th legal action in ascending order,
+ * j = mulhi64(word, k).  games: device int32 [rows], the game each row belongs to, or NULL = the row index.  count: device
+ * int32 [1], the compact leaf count (rows at or past it are not written), or NULL = all rows.  Connect4 n = 4..8 and
+ * TicTacToe n = 3..5; playouts in [1, 4096]; anything else, and null pointers with rows > 0, is refused (AZG_ERR_INVALID). */
+int azg_rollout_eval(int game, int n, const uint64_t* states, const int32_t* games, int64_t rows, const int32_t* count,
+                     int playouts, uint64_t seed, float* pi, float* v, azg_stream stream);
 int azg_arena_action_size(const azg_arena* a);
 /* new MCTS object for the listed games (Coach.py:96): clear their tables.  game_ids: device
  * int32 [count], or NULL = all games. */
